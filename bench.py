@@ -12,11 +12,14 @@ whole genome with the CLI's own --step flag: every S-th informative site is a ce
 the full 10 M-site data, exactly like `-s S` in the reference (v1:603-608).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          # this repo, CUDA
+    python bench.py --dump-outputs DIR [...]                      # also write the rows of the last timed step
+                                                                  # (CUDA arm only: the reference arm has no timed rows)
     python bench.py --impl reference [...]                        # CPU arm: the reference's own path on host cores
                                                                   # (C port on every step + the unmodified script once)
 
 Every CUDA run carries a parity gate: rows of the timed scan are compared with the CPU oracle
-(`parity` in the JSON line) and the run fails on a mismatch.
+(`parity` in the JSON line) and the run fails on a mismatch.  The synthetic genome and the centre list are
+seeded, so two builds run with the same arguments scan the same inputs and their dumps compare row for row.
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
 """
@@ -52,6 +55,7 @@ FLOP_BLOCK = FLOP_EXP + 32 * (10.0 + 2.0)   # far field, per unit visit: one exp
                                             # ten multiplications (power by squaring) and one FMA
 FLOP_EDGE = 9.0            # far field: five moments of a block-remainder site (besides its exp)
 FLOP_POLY = 2.0            # far field: one Horner FMA per polynomial term and grid point
+DUMP_BYTES = 60_000_000    # --dump-outputs: array data per run, so that the files with their headers stay within 64 MB
 
 
 def algorithmic_flops(cnt, n_xa, n_items):
@@ -222,6 +226,21 @@ def run_cpu_oracle(problems, plans, sample, threads, report_all=False, keep=None
         if keep is not None:
             keep.append((c, idx, res))
     return time.perf_counter() - t0, centres, pairs
+
+
+def dump_outputs(out_dir, rows, limit=DUMP_BYTES):
+    """Write the rows one step returns, (T, iA, ix, ia, nsites) per centre in global centre order, as
+    <out_dir>/<field>.npy in float64 (exact for the int32 fields), with centre.npy: the index of each row.
+    Rows beyond `limit` bytes are replaced by a fixed, seeded sample of the centres."""
+    fields = [np.asarray(a, dtype=np.float64) for a in rows]
+    n = len(fields[0])
+    per_row = 8 * (len(fields) + 1)
+    keep = np.arange(n)
+    if n * per_row > limit:
+        keep = np.sort(np.random.default_rng(0).choice(n, limit // per_row, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in zip(('centre', 'T', 'iA', 'ix', 'ia', 'nsites'), [keep.astype(np.float64)] + fields):
+        np.save(os.path.join(out_dir, name + '.npy'), a if name == 'centre' else a[keep])
 
 
 def parity_sample(plans, T_rows, n_positive=64, n_any=32):
@@ -597,6 +616,8 @@ def cuda_arm(opt, rank, world, local_rank):
     pairs_all, launches_all = (int(v) for v in reduce_sum([cnt['pairs'], cnt['launches']]))
     value = total_centres * n_grid * opt.steps / (ms * 1e-3)
     resident_rows = sharding.unpack_rows(gathered.cpu(), torch) if rank == 0 else None
+    if rank == 0 and opt.dump_outputs:
+        dump_outputs(opt.dump_outputs, [a.numpy() for a in resident_rows])
 
     # the same workload with every site evaluated directly (option farfield = 0): the FP64-bound kernel
     direct = None
@@ -792,7 +813,14 @@ def main():
                     help='reference arm: skip the run of the unmodified script (oracle/_ref)')
     ap.add_argument('--profile', action='store_true',
                     help='only the device-resident timed steps (for ncu): no direct / e2e / strong legs')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the rows of the last timed step to DIR/<field>.npy; CUDA arm only, '
+                         'refused with --impl reference')
     opt = ap.parse_args()
+    if opt.steps < 1 or opt.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if opt.dump_outputs and opt.impl != 'cuda':
+        ap.error('--dump-outputs writes the rows of the CUDA arm')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))

@@ -1,5 +1,7 @@
 """bench.py's host logic (no GPU): the parity gate must fail on a wrong row, the centre sample must contain the
-rows that carry a real maximum, and the flop accounting must add up."""
+rows that carry a real maximum, the output dump must hold the rows, and the flop accounting must add up."""
+import os
+
 import numpy as np
 
 import bench
@@ -46,6 +48,23 @@ def test_parity_gate_passes_on_equal_rows_and_fails_on_any_difference():
     wrong = [a.copy() for a in rows_all]
     wrong[0][0] += 1.0
     assert not bench.parity_check([_P(), _P()], kept_all, bounds, rows, tuple(wrong))['ok']
+
+
+def test_dump_outputs_writes_every_row_or_a_fixed_sample(tmp_path):
+    rows = _fake(n=1000)
+    bench.dump_outputs(str(tmp_path / 'all'), rows)
+    got = {f: np.load(tmp_path / 'all' / f'{f}.npy') for f in ('centre', 'T', 'iA', 'ix', 'ia', 'nsites')}
+    assert all(a.dtype == np.float64 and a.shape == (1000,) for a in got.values())
+    assert np.array_equal(got['centre'], np.arange(1000))
+    for f, a in zip(('T', 'iA', 'ix', 'ia', 'nsites'), rows):
+        assert np.array_equal(got[f], a)
+    limit = 48 * 300                                          # room for 300 rows of the six fields
+    for run in ('s1', 's2'):
+        bench.dump_outputs(str(tmp_path / run), rows, limit=limit)
+    c1, c2 = (np.load(tmp_path / run / 'centre.npy') for run in ('s1', 's2'))
+    assert len(c1) == 300 and np.array_equal(c1, c2) and np.all(np.diff(c1) > 0)
+    assert np.array_equal(np.load(tmp_path / 's1' / 'T.npy'), rows[0][c1.astype(np.int64)])
+    assert sum(os.path.getsize(p) for p in (tmp_path / 's1').iterdir()) <= limit + 6 * 128
 
 
 def test_flop_accounting():
