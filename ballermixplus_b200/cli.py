@@ -2,7 +2,8 @@
 
 Same flags, defaults, precedence and console messages as the reference's ``main``
 (/root/reference/BalLeRMix+_v1.py:715-802); one extra flag, ``--device``, picks the
-GPU.  Differences, all on paths where the reference raises (SURVEY.md appendix A.2,
+GPU, and ``--support`` / ``--supportDrop`` write support intervals of A_hat, x_hat and s_hat (support.py).
+Differences, all on paths where the reference raises (SURVEY.md appendix A.2,
 DESIGN.md "flags without a reference behaviour"): ``--rangeA``, ``--findPos`` and
 ``--minCount`` with ``--noFreq`` work here.
 """
@@ -17,6 +18,7 @@ from .inputs import InputData
 from .neutral import NeutralSFS
 from .scan import Scan
 from .selection import NormalizedBetaBinom
+from .support import DEFAULT_DROP, check_drop
 
 
 def build_parser():
@@ -61,7 +63,22 @@ def build_parser():
     p.add_argument('--rangeA', dest='seqA', help='<Amin>,<Amax>,<Astep> grid for the linkage parameter A.')
     p.add_argument('--listA', dest='listA', help='Comma-separated list of A values.')
     p.add_argument('--device', dest='device', type=int, default=0, help='CUDA device to run the scan on.')
+    p.add_argument('--support', dest='support', default=None,
+                   help='Also write FILE: per output row, the lowest and highest A, x and s whose profile '
+                        'likelihood is within --supportDrop of the row\'s CLR. These are support intervals of a '
+                        'composite likelihood: sites are not independent, so they are not calibrated confidence '
+                        'intervals. One GPU only (not under torchrun).')
+    p.add_argument('--supportDrop', dest='supportDrop', type=_drop, default=DEFAULT_DROP,
+                   help='Drop in T = 2 log LR units that defines the --support intervals. Default '
+                        f'{DEFAULT_DROP} (the chi-square(1) 0.95 quantile).')
     return p
+
+
+def _drop(text):
+    try:
+        return check_drop(text)
+    except ValueError as exc:
+        raise argparse.ArgumentTypeError(str(exc)) from None
 
 
 def main(argv=None):
@@ -73,6 +90,8 @@ def main(argv=None):
         parser.print_help()
         sys.exit()
     opt = parser.parse_args(argv)
+    if opt.support is not None and int(os.environ.get('WORLD_SIZE', '1')) > 1:
+        parser.error('--support runs on one GPU; launch without torchrun (WORLD_SIZE > 1)')
 
     if opt.getSpec:
         print('You\'ve chosen to generate site frequency spectrum...')
@@ -103,7 +122,8 @@ def main(argv=None):
 
     print('\n%s. Start computing likelihood raito...' % (datetime.now()))
     Scan(data, Neutral, Sel_Probs, grid, opt.outfile, fixSize=opt.size, r=opt.w, s=opt.step,
-         phys=opt.phys, noCenter=opt.noCenter, device=opt.device)
+         phys=opt.phys, noCenter=opt.noCenter, device=opt.device, support=opt.support,
+         support_drop=opt.supportDrop)
     print(f'\n{datetime.now()}. Pipeline finished.')
 
 

@@ -17,7 +17,7 @@ ABI_SYMBOLS = (
     'blmx_abi_version', 'blmx_last_error', 'blmx_device_count', 'blmx_create', 'blmx_destroy',
     'blmx_load', 'blmx_scan', 'blmx_scan_device', 'blmx_scan_oneshot', 'blmx_set_option',
     'blmx_last_counters', 'blmx_last_counters6', 'blmx_last_counters8', 'blmx_problem_info',
-    'blmx_last_kernel_ms', 'blmx_measure_fp64_peak',
+    'blmx_last_kernel_ms', 'blmx_measure_fp64_peak', 'blmx_scan_profile', 'blmx_scan_surface',
 )
 
 
@@ -34,6 +34,10 @@ class Problem(C.Structure):
 class Result(C.Structure):
     _fields_ = [('T', C.c_void_p), ('iA', C.c_void_p), ('ix', C.c_void_p), ('ia', C.c_void_p),
                 ('nsites', C.c_void_p)]
+
+
+class Profile(C.Structure):
+    _fields_ = [('TA', C.c_void_p), ('Tx', C.c_void_p), ('Ta', C.c_void_p), ('nsA', C.c_void_p)]
 
 
 _lib = None
@@ -53,6 +57,10 @@ def lib():
         L.blmx_load.argtypes = [C.c_void_p, C.POINTER(Problem)]
         L.blmx_scan.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.POINTER(Result)]
+        L.blmx_scan_profile.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.POINTER(Result), C.POINTER(Profile)]
+        L.blmx_scan_surface.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_void_p]
         L.blmx_scan_device.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.POINTER(Result), C.c_void_p]
         L.blmx_scan_oneshot.argtypes = [C.c_int, C.POINTER(Problem), C.c_int64, C.c_void_p,
@@ -140,19 +148,57 @@ class Scanner:
         _check(lib().blmx_load(self._h, C.byref(st)))
         return self
 
-    def scan(self, t, lo, hi):
-        """HOST arrays in, HOST arrays out (H2D + kernels + D2H, synchronous)."""
+    @staticmethod
+    def _centres(t, lo, hi):
         t = np.ascontiguousarray(t, dtype=np.float64)
         lo = np.ascontiguousarray(lo, dtype=np.int64)
         hi = np.ascontiguousarray(hi, dtype=np.int64)
-        n = len(t)
-        if len(lo) != n or len(hi) != n:
+        if len(lo) != len(t) or len(hi) != len(t):
             raise ValueError('t, lo, hi differ in length')
+        return t, lo, hi
+
+    def _grid(self):
+        p = getattr(self, '_problem', None)
+        if p is None:
+            raise BlmxError('no problem loaded')
+        return len(p.A), p.n_x, p.n_a
+
+    def scan(self, t, lo, hi):
+        """HOST arrays in, HOST arrays out (H2D + kernels + D2H, synchronous)."""
+        t, lo, hi = self._centres(t, lo, hi)
+        n = len(t)
         T = np.zeros(n, np.float64)
         iA, ix, ia, ns = (np.full(n, -1, np.int32) for _ in range(4))
         res = Result(_ptr(T), _ptr(iA), _ptr(ix), _ptr(ia), _ptr(ns))
         _check(lib().blmx_scan(self._h, n, _ptr(t), _ptr(lo), _ptr(hi), C.byref(res)))
         return T, iA, ix, ia, ns
+
+    def scan_profile(self, t, lo, hi):
+        """``scan`` plus the profiles of the likelihood surface (blmx_scan_profile):
+        -> (T, iA, ix, ia, nsites, TA [n, n_A], Tx [n, n_x], Ta [n, n_a], nsA [n, n_A])."""
+        t, lo, hi = self._centres(t, lo, hi)
+        n = len(t)
+        n_A, n_x, n_a = self._grid()
+        T = np.zeros(n, np.float64)
+        iA, ix, ia, ns = (np.full(n, -1, np.int32) for _ in range(4))
+        TA, Tx, Ta = np.empty((n, n_A)), np.empty((n, n_x)), np.empty((n, n_a))
+        nsA = np.zeros((n, n_A), np.int32)
+        res = Result(_ptr(T), _ptr(iA), _ptr(ix), _ptr(ia), _ptr(ns))
+        prof = Profile(_ptr(TA), _ptr(Tx), _ptr(Ta), _ptr(nsA))
+        _check(lib().blmx_scan_profile(self._h, n, _ptr(t), _ptr(lo), _ptr(hi), C.byref(res), C.byref(prof)))
+        return T, iA, ix, ia, ns, TA, Tx, Ta, nsA
+
+    def scan_surface(self, t, lo, hi):
+        """The whole likelihood surface (blmx_scan_surface) -> (S [n, n_A, n_x, n_a], nsA [n, n_A]).
+        S is T at every grid point; -inf everywhere for an A without sites.  n * n_A * n_x * n_a doubles come
+        back to the host: meant for a few centres."""
+        t, lo, hi = self._centres(t, lo, hi)
+        n = len(t)
+        n_A, n_x, n_a = self._grid()
+        S = np.empty((n, n_A, n_x, n_a))
+        nsA = np.zeros((n, n_A), np.int32)
+        _check(lib().blmx_scan_surface(self._h, n, _ptr(t), _ptr(lo), _ptr(hi), _ptr(S), _ptr(nsA)))
+        return S, nsA
 
     def scan_device(self, n, d_t, d_lo, d_hi, d_T, d_iA, d_ix, d_ia, d_ns, stream=0):
         """Raw DEVICE pointers (ints) in and out, asynchronous on `stream`."""

@@ -11,7 +11,7 @@ from datetime import datetime
 
 import numpy as np
 
-from . import fastio, windows
+from . import fastio, support as support_mod, windows
 from .native import Scanner
 from .problem import build_problem
 
@@ -31,6 +31,14 @@ class DeviceScan:
     def run(self, t, lo, hi):
         """-> (T float64[n], iA, ix, ia, nsites int32[n]); indices into the visiting order."""
         return self.scanner.scan(t, lo, hi)
+
+    def run_profile(self, t, lo, hi):
+        """``run`` plus the profiles of the likelihood surface -> (T, iA, ix, ia, nsites, TA, Tx, Ta, nsA)."""
+        return self.scanner.scan_profile(t, lo, hi)
+
+    def surface(self, t, lo, hi):
+        """The whole likelihood surface of a few centres -> (S [n, n_A, n_x, n_a], nsA [n, n_A])."""
+        return self.scanner.scan_surface(t, lo, hi)
 
     def run_device(self, t, lo, hi, torch, device):
         """Same scan with the centres uploaded once and the results LEFT ON THE DEVICE as torch tensors
@@ -176,15 +184,44 @@ def scan_rows_multi_gpu(dev, t, lo, hi, rank, world, local_rank):
             dist.destroy_process_group()
 
 
+#: centres per blmx_scan_profile call of ``Scan(..., support=...)``: bounds the host memory of the profiles
+SUPPORT_CHUNK = 65536
+
+
+def scan_with_support(dev, t, lo, hi, q):
+    """The rows of ``dev.run`` plus their support intervals (support.py), scanned in chunks of centres so that
+    only the intervals of a genome-sized run stay in host memory -> (rows, intervals)."""
+    n = len(t)
+    rows = [np.zeros(n), *(np.full(n, -1, np.int32) for _ in range(3)), np.zeros(n, np.int32)]
+    iv = {k: np.full(n, -1, np.int32) for k in ('A_lo', 'A_hi', 'x_lo', 'x_hi', 's_lo', 's_hi')}
+    for b in range(0, n, SUPPORT_CHUNK):
+        e = min(n, b + SUPPORT_CHUNK)
+        T, iA, ix, ia, ns, TA, Tx, Ta, _ = dev.run_profile(t[b:e], lo[b:e], hi[b:e])
+        for col, v in zip(rows, (T, iA, ix, ia, ns)):
+            col[b:e] = v
+        for k, v in support_mod.support_intervals(T, iA, TA, Tx, Ta, dev.order, q).items():
+            iv[k][b:e] = v
+    return tuple(rows), iv
+
+
 class Scan:
     """Same constructor as the reference class (v1:613); runs the scan and writes ``outfile``.
 
     Launched under ``torchrun --nproc-per-node N`` the centres are sharded over N GPUs and rank 0
-    writes the file (the other ranks write nothing)."""
+    writes the file (the other ranks write nothing).
+
+    ``support`` (a path): also write, per row of ``outfile``, the support intervals of A_hat, x_hat and
+    s_hat at a drop of ``support_drop`` in T units (support.py: intervals of a composite likelihood, not
+    calibrated confidence intervals).  One GPU only."""
 
     def __init__(self, InputData, NeutralSFS, NormalizedBetaBinom, Grids, outfile, fixSize=False,
-                 r=0, s=1, phys=False, noCenter=False, device=0):
+                 r=0, s=1, phys=False, noCenter=False, device=0, support=None,
+                 support_drop=support_mod.DEFAULT_DROP):
         rank, world, local_rank = _world()
+        if support is not None:
+            support_drop = support_mod.check_drop(support_drop)
+            if world > 1:
+                raise ValueError('--support runs on one GPU: launch without torchrun (WORLD_SIZE > 1)')
         plan = windows.make_plan(InputData, fixSize=fixSize, r=r, s=s, phys=phys, noCenter=noCenter)
         if rank == 0:
             print('writing output to %s' % (outfile))
@@ -192,6 +229,9 @@ class Scan:
             # must fail now, not after the scan
             with open(outfile, 'w'):
                 pass
+            if support is not None:
+                with open(support, 'w'):
+                    pass
         if world > 1:
             from .native import device_count
             device = local_rank % max(1, device_count())
@@ -201,9 +241,14 @@ class Scan:
             live = np.flatnonzero(~gap)
             T = np.zeros(len(plan)); iA = np.full(len(plan), -1, np.int32)
             ix = iA.copy(); ia = iA.copy(); ns = np.zeros(len(plan), np.int32)
+            iv = {k: np.full(len(plan), -1, np.int32) for k in ('A_lo', 'A_hi', 'x_lo', 'x_hi', 's_lo', 's_hi')}
             if len(live):
                 if world > 1:
                     got = scan_rows_multi_gpu(dev, t[live], lo[live], hi[live], rank, world, local_rank)
+                elif support is not None:
+                    got, got_iv = scan_with_support(dev, t[live], lo[live], hi[live], support_drop)
+                    for k, v in got_iv.items():
+                        iv[k][live] = v
                 else:
                     got = dev.run(t[live], lo[live], hi[live])
                 if got is not None:
@@ -211,6 +256,11 @@ class Scan:
             self.results = (T, iA, ix, ia, ns) if rank == 0 else None
             if rank == 0:
                 write_scan(outfile, plan, dev.order, T, iA, ix, ia, ns)
+                if support is not None:
+                    self.support = iv
+                    with open(support, 'w') as fh:
+                        fh.write(support_mod.SUPPORT_HEADER)
+                        fh.writelines(support_mod.format_support(plan, dev.order, T, iA, ix, ia, ns, iv))
         finally:
             dev.close()
         if rank == 0:

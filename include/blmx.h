@@ -114,6 +114,39 @@ int blmx_scan(blmx_handle *h, int64_t n_centres, const double *t, const int64_t 
 int blmx_scan_device(blmx_handle *h, int64_t n_centres, const double *d_t, const int64_t *d_lo,
                      const int64_t *d_hi, const blmx_result *d_out, void *cuda_stream);
 
+/*
+ * The likelihood surface and its profiles.
+ *
+ * The surface of centre j is T(A, x, a) = 2*(sum log mix - sum log g) (v1:499) at every grid point, the value
+ * the maximum of the rows is taken over.  An A with no site in the window (nsites = 0, which the reference
+ * skips, v1:458) has T = -inf at every grid point.  T may be NaN or -inf where the tables make it so.
+ *
+ * The profiles of centre j are maxima of its surface over all but one grid axis, over the A with sites only:
+ *   TA[j][iA] = max over (x, a),   Tx[j][ix] = max over (A, a),   Ta[j][ia] = max over (A, x),
+ * and nsA[j][iA] = sites used at A.  NaN never wins a maximum (the strict '>' of v1:501); an entry with
+ * nothing to take is -inf.  Profiles do not depend on option "report_all": they are never clamped at 0.
+ * Indices are visiting-order indices, as in blmx_result; every array is row-major per centre, centres in the
+ * order of the call.
+ *
+ * Both calls take HOST buffers and are synchronous, like blmx_scan.  The library stages the surface through
+ * device scratch of at most 1 GiB per launch (fewer centres per launch than option "batch" when n_A*n_x*n_a
+ * is large).
+ */
+typedef struct {
+    double  *TA;       /* [n_centres][n_A] */
+    double  *Tx;       /* [n_centres][n_x] */
+    double  *Ta;       /* [n_centres][n_a] */
+    int32_t *nsA;      /* [n_centres][n_A] */
+} blmx_profile;
+
+/* blmx_scan plus the profiles: `out` gets exactly what blmx_scan writes (report_all included). */
+int blmx_scan_profile(blmx_handle *h, int64_t n_centres, const double *t, const int64_t *lo,
+                      const int64_t *hi, const blmx_result *out, const blmx_profile *prof);
+
+/* The full surface of a few centres (for plots and tests): S[j][iA][ix*n_a + ia], nsA[j][iA]. */
+int blmx_scan_surface(blmx_handle *h, int64_t n_centres, const double *t, const int64_t *lo,
+                      const int64_t *hi, double *S, int32_t *nsA);
+
 /* One-shot form of the seam: create + load + scan + destroy on `device`. */
 int blmx_scan_oneshot(int device, const blmx_problem *p, int64_t n_centres, const double *t,
                       const int64_t *lo, const int64_t *hi, const blmx_result *out);
