@@ -16,7 +16,7 @@ LIB_PATH = os.environ.get('BLMX_LIB') or os.path.join(_HERE, 'libblmx.so')   # B
 ABI_SYMBOLS = (
     'blmx_abi_version', 'blmx_last_error', 'blmx_device_count', 'blmx_create', 'blmx_destroy',
     'blmx_load', 'blmx_scan', 'blmx_scan_device', 'blmx_scan_oneshot', 'blmx_set_option',
-    'blmx_last_counters', 'blmx_last_counters6', 'blmx_last_counters8', 'blmx_problem_info',
+    'blmx_last_counters', 'blmx_last_counters6', 'blmx_last_counters8', 'blmx_last_counters9', 'blmx_problem_info',
     'blmx_last_kernel_ms', 'blmx_measure_fp64_peak', 'blmx_scan_profile', 'blmx_scan_surface',
 )
 
@@ -70,6 +70,7 @@ def lib():
                                          C.POINTER(C.c_uint64)]
         L.blmx_last_counters6.argtypes = [C.c_void_p, C.POINTER(C.c_uint64 * 6), C.POINTER(C.c_uint64)]
         L.blmx_last_counters8.argtypes = [C.c_void_p, C.POINTER(C.c_uint64 * 8), C.POINTER(C.c_uint64)]
+        L.blmx_last_counters9.argtypes = [C.c_void_p, C.POINTER(C.c_uint64 * 9), C.POINTER(C.c_uint64)]
         L.blmx_problem_info.argtypes = [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64),
                                         C.POINTER(C.c_int64)]
         L.blmx_last_kernel_ms.argtypes = [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int64)]
@@ -213,11 +214,12 @@ class Scanner:
         return a.value, c.value
 
     def counters_all(self):
-        """dict of the work counters of the most recent scan (see blmx_last_counters8)."""
-        v, c = (C.c_uint64 * 8)(), C.c_uint64(0)
-        _check(lib().blmx_last_counters8(self._h, C.byref(v), C.byref(c)))
+        """dict of the work counters of the most recent scan (see blmx_last_counters9)."""
+        v, c = (C.c_uint64 * 9)(), C.c_uint64(0)
+        _check(lib().blmx_last_counters9(self._h, C.byref(v), C.byref(c)))
         return {'pairs': v[0], 'single': v[1], 'far_blocks': v[2], 'far_terms': v[3], 'far_sites': v[4],
-                'range_violations': v[5], 'edge_sites': v[6], 'quads': v[7], 'launches': c.value}
+                'range_violations': v[5], 'edge_sites': v[6], 'quads': v[7], 'pruned_items': v[8],
+                'launches': c.value}
 
     def problem_info(self):
         """Far-field layout of the loaded problem: whole blocks, sites per block, bytes of moments in HBM."""

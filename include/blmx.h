@@ -166,6 +166,11 @@ int blmx_scan_oneshot(int device, const blmx_problem *p, int64_t n_centres, cons
  *                T and argmax on every centre instead of the all-zero row
  *   "batch"      centres per kernel launch (scratch = batch * n_A * 16 bytes)
  *   "timing"     1 = record CUDA events around every scan kernel (see blmx_last_kernel_ms)
+ *   "prune"      1 (default) = before the scan kernel, prove from an upper bound on T which (centre, A) items
+ *                have T <= 0 at every grid point and skip their exact evaluation (their candidate is the
+ *                all-zero one whatever their exact T, so the rows do not change); 0 = evaluate every item.
+ *                Only the default scan prunes: not with report_all, surfaces or profiles, group 1,
+ *                farfield 0, unsorted positions or class rows with inf/nan
  */
 int blmx_set_option(blmx_handle *h, const char *name, int64_t value);
 
@@ -186,6 +191,9 @@ int blmx_last_counters(blmx_handle *h, uint64_t *site_pairs, uint64_t *single_pa
  * sites on every grid point). */
 int blmx_last_counters6(blmx_handle *h, uint64_t *six, uint64_t *launches);
 int blmx_last_counters8(blmx_handle *h, uint64_t *eight, uint64_t *launches);
+/* [0..7] as blmx_last_counters8, [8] items proved T <= 0 everywhere and skipped (option "prune"); their sites
+ * are counted in [0] and, as they are not multiplied in per grid point, also in [4]. */
+int blmx_last_counters9(blmx_handle *h, uint64_t *nine, uint64_t *launches);
 
 /* Far-field layout of the loaded problem: whole blocks, sites per block, bytes of block moments
  * resident on the device (0 blocks: every site is evaluated directly). */
