@@ -2,7 +2,8 @@
 
 Same flags, defaults, precedence and console messages as the reference's ``main``
 (/root/reference/BalLeRMix+_v1.py:715-802); one extra flag, ``--device``, picks the
-GPU, and ``--support`` / ``--supportDrop`` write support intervals of A_hat, x_hat and s_hat (support.py).
+GPU, ``--support`` / ``--supportDrop`` write support intervals of A_hat, x_hat and s_hat (support.py), and
+``--null`` / ``--pvalues`` write empirical p-values from scans of neutral replicates (null.py).
 Differences, all on paths where the reference raises (SURVEY.md appendix A.2,
 DESIGN.md "flags without a reference behaviour"): ``--rangeA``, ``--findPos`` and
 ``--minCount`` with ``--noFreq`` work here.
@@ -16,6 +17,7 @@ from .grids import Grids
 from .helpers import getConfig, getSpect
 from .inputs import InputData
 from .neutral import NeutralSFS
+from .null import read_list
 from .scan import Scan
 from .selection import NormalizedBetaBinom
 from .support import DEFAULT_DROP, check_drop
@@ -71,6 +73,16 @@ def build_parser():
     p.add_argument('--supportDrop', dest='supportDrop', type=_drop, default=DEFAULT_DROP,
                    help='Drop in T = 2 log LR units that defines the --support intervals. Default '
                         f'{DEFAULT_DROP} (the chi-square(1) 0.95 quantile).')
+    p.add_argument('--null', dest='null', default=None,
+                   help='Text file listing neutral replicate inputs, one path per line (relative to the list; '
+                        'blank and # lines skipped). Every replicate is scanned with exactly the flags and '
+                        '--spect of this run, and --pvalues gets each row\'s empirical p-value against the '
+                        'pooled replicate CLRs, p = (1 + #{null >= CLR}) / (1 + N_null). The p-values are only as '
+                        'good as the neutral model the replicates were simulated under, and they are not '
+                        'corrected for multiple testing (the printed quantiles of the per-replicate maximum CLR '
+                        'give a region-level threshold). Needs --pvalues.')
+    p.add_argument('--pvalues', dest='pvalues', default=None,
+                   help='With --null: write FILE with physPos, genPos, CLR and p_value per output row.')
     return p
 
 
@@ -92,6 +104,13 @@ def main(argv=None):
     opt = parser.parse_args(argv)
     if opt.support is not None and int(os.environ.get('WORLD_SIZE', '1')) > 1:
         parser.error('--support runs on one GPU; launch without torchrun (WORLD_SIZE > 1)')
+    if (opt.null is None) != (opt.pvalues is None):
+        parser.error('--null and --pvalues must be given together')
+    if opt.null is not None:
+        try:
+            read_list(opt.null)             # a bad list fails before any input is read
+        except (OSError, ValueError) as exc:
+            parser.error(str(exc))
 
     if opt.getSpec:
         print('You\'ve chosen to generate site frequency spectrum...')
@@ -123,7 +142,7 @@ def main(argv=None):
     print('\n%s. Start computing likelihood raito...' % (datetime.now()))
     Scan(data, Neutral, Sel_Probs, grid, opt.outfile, fixSize=opt.size, r=opt.w, s=opt.step,
          phys=opt.phys, noCenter=opt.noCenter, device=opt.device, support=opt.support,
-         support_drop=opt.supportDrop)
+         support_drop=opt.supportDrop, null=opt.null, pvalues=opt.pvalues)
     print(f'\n{datetime.now()}. Pipeline finished.')
 
 

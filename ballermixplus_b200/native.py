@@ -18,6 +18,7 @@ ABI_SYMBOLS = (
     'blmx_load', 'blmx_scan', 'blmx_scan_device', 'blmx_scan_oneshot', 'blmx_set_option',
     'blmx_last_counters', 'blmx_last_counters6', 'blmx_last_counters8', 'blmx_last_counters9', 'blmx_problem_info',
     'blmx_last_kernel_ms', 'blmx_measure_fp64_peak', 'blmx_scan_profile', 'blmx_scan_surface',
+    'blmx_load_segmented',
 )
 
 
@@ -55,6 +56,7 @@ def lib():
         L.blmx_create.argtypes = [C.c_int, C.POINTER(C.c_void_p)]
         L.blmx_destroy.argtypes = [C.c_void_p]
         L.blmx_load.argtypes = [C.c_void_p, C.POINTER(Problem)]
+        L.blmx_load_segmented.argtypes = [C.c_void_p, C.POINTER(Problem), C.c_int64, C.c_void_p]
         L.blmx_scan.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.POINTER(Result)]
         L.blmx_scan_profile.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
@@ -103,9 +105,13 @@ def measure_fp64_peak(device=0, seconds=0.5):
 
 
 class ScanProblem:
-    """Host arrays of one blmx_problem (see include/blmx.h for the meaning of each)."""
+    """Host arrays of one blmx_problem (see include/blmx.h for the meaning of each).
 
-    def __init__(self, genpos, cls, G, SP, A, n_x, n_a):
+    ``seg_start`` (optional): first site of each segment of a problem made of several sequences laid end to
+    end (blmx_load_segmented); ``Scanner.load`` then loads it segmented."""
+
+    def __init__(self, genpos, cls, G, SP, A, n_x, n_a, seg_start=None):
+        self.seg_start = None if seg_start is None else np.ascontiguousarray(seg_start, dtype=np.int64)
         self.genpos = np.ascontiguousarray(genpos, dtype=np.float64)
         self.cls = np.ascontiguousarray(cls, dtype=np.int32)
         self.G = np.ascontiguousarray(G, dtype=np.float64)
@@ -146,7 +152,11 @@ class Scanner:
     def load(self, problem):
         self._problem = problem          # keep the host arrays alive during the call
         st = problem.as_struct()
-        _check(lib().blmx_load(self._h, C.byref(st)))
+        seg = getattr(problem, 'seg_start', None)
+        if seg is None:
+            _check(lib().blmx_load(self._h, C.byref(st)))
+        else:
+            _check(lib().blmx_load_segmented(self._h, C.byref(st), len(seg), _ptr(seg)))
         return self
 
     @staticmethod

@@ -11,7 +11,7 @@ from datetime import datetime
 
 import numpy as np
 
-from . import fastio, support as support_mod, windows
+from . import fastio, null as null_mod, support as support_mod, windows
 from .native import Scanner
 from .problem import build_problem
 
@@ -23,7 +23,17 @@ class DeviceScan:
 
     def __init__(self, InputData, NeutralSFS, NormalizedBetaBinom, Grids, device=0, group=None,
                  farfield=None):
-        self.problem, self.order = build_problem(InputData, NeutralSFS, NormalizedBetaBinom, Grids)
+        self._start(*build_problem(InputData, NeutralSFS, NormalizedBetaBinom, Grids), device, group, farfield)
+
+    @classmethod
+    def from_problem(cls, problem, order, device=0, group=None, farfield=None):
+        """A ScanProblem built elsewhere (a segmented one: null.py) and its GridOrder."""
+        self = cls.__new__(cls)
+        self._start(problem, order, device, group, farfield)
+        return self
+
+    def _start(self, problem, order, device, group, farfield):
+        self.problem, self.order = problem, order
         if farfield is None and os.environ.get('BLMX_FARFIELD'):
             farfield = int(os.environ['BLMX_FARFIELD'])
         self.scanner = Scanner(device=device, group=group, farfield=farfield).load(self.problem)
@@ -142,12 +152,13 @@ def ranks_own_a_gpu():
     return device_count() >= _local_world()
 
 
-def scan_rows_multi_gpu(dev, t, lo, hi, rank, world, local_rank):
+def scan_rows_multi_gpu(dev, t, lo, hi, rank, world, local_rank, keep_group=False):
     """One process per GPU (torchrun): every rank scans a cost-balanced contiguous slice of the centres,
     one gather brings the rows to rank 0 (sharding.py).  When every rank of the node has its own GPU the rows
     stay on the device from the scan kernel to the NCCL gather (``DeviceScan.run_device``); when several ranks
     share one device (tests on a one-GPU box) the gather runs over gloo on host tensors.  Returns the five
-    result arrays on rank 0 and None elsewhere."""
+    result arrays on rank 0 and None elsewhere.  ``keep_group``: leave the process group this call starts
+    running for a later scan (``end_group`` ends it)."""
     import torch
     import torch.distributed as dist
     from . import sharding
@@ -174,14 +185,23 @@ def scan_rows_multi_gpu(dev, t, lo, hi, rank, world, local_rank):
 
     ok = False
     try:
-        got = sharding.scan_sharded(dev.problem.genpos, dev.problem.A, t, lo, hi, rank, world, scan_fn, dist, torch)
+        got = sharding.scan_sharded(dev.problem.genpos, dev.problem.A, t, lo, hi, rank, world, scan_fn, dist, torch,
+                                    seg_start=getattr(dev.problem, 'seg_start', None))
         ok = True
         return None if got is None else tuple(a.cpu().numpy() for a in got)
     finally:
-        if started:
+        if started and not (ok and keep_group):
             if ok:                      # a rank that failed must not wait for the others (they would hang with it)
                 dist.barrier()
             dist.destroy_process_group()
+
+
+def end_group():
+    """End the process group a ``scan_rows_multi_gpu(..., keep_group=True)`` left running."""
+    import torch.distributed as dist
+    if dist.is_initialized():
+        dist.barrier()
+        dist.destroy_process_group()
 
 
 #: centres per blmx_scan_profile call of ``Scan(..., support=...)``: bounds the host memory of the profiles
@@ -212,16 +232,22 @@ class Scan:
 
     ``support`` (a path): also write, per row of ``outfile``, the support intervals of A_hat, x_hat and
     s_hat at a drop of ``support_drop`` in T units (support.py: intervals of a composite likelihood, not
-    calibrated confidence intervals).  One GPU only."""
+    calibrated confidence intervals).  One GPU only.
+
+    ``null`` (a replicate list) and ``pvalues`` (a path), given together: also scan the neutral replicates the
+    list names with the same flags and tables, as one segmented problem, and write, per row of ``outfile``,
+    its empirical p-value against the pooled null CLRs (null.py).  ``outfile`` is the same either way."""
 
     def __init__(self, InputData, NeutralSFS, NormalizedBetaBinom, Grids, outfile, fixSize=False,
                  r=0, s=1, phys=False, noCenter=False, device=0, support=None,
-                 support_drop=support_mod.DEFAULT_DROP):
+                 support_drop=support_mod.DEFAULT_DROP, null=None, pvalues=None):
         rank, world, local_rank = _world()
         if support is not None:
             support_drop = support_mod.check_drop(support_drop)
             if world > 1:
                 raise ValueError('--support runs on one GPU: launch without torchrun (WORLD_SIZE > 1)')
+        if (null is None) != (pvalues is None):
+            raise ValueError('--null and --pvalues go together')
         plan = windows.make_plan(InputData, fixSize=fixSize, r=r, s=s, phys=phys, noCenter=noCenter)
         if rank == 0:
             print('writing output to %s' % (outfile))
@@ -232,6 +258,13 @@ class Scan:
             if support is not None:
                 with open(support, 'w'):
                     pass
+            if pvalues is not None:
+                with open(pvalues, 'w'):
+                    pass
+        setup = None
+        if null is not None:
+            setup = null_mod.NullSetup(null, InputData, NeutralSFS, NormalizedBetaBinom, Grids, fixSize=fixSize,
+                                       r=r, s=s, phys=phys, noCenter=noCenter)
         if world > 1:
             from .native import device_count
             device = local_rank % max(1, device_count())
@@ -244,7 +277,8 @@ class Scan:
             iv = {k: np.full(len(plan), -1, np.int32) for k in ('A_lo', 'A_hi', 'x_lo', 'x_hi', 's_lo', 's_hi')}
             if len(live):
                 if world > 1:
-                    got = scan_rows_multi_gpu(dev, t[live], lo[live], hi[live], rank, world, local_rank)
+                    got = scan_rows_multi_gpu(dev, t[live], lo[live], hi[live], rank, world, local_rank,
+                                              keep_group=setup is not None)
                 elif support is not None:
                     got, got_iv = scan_with_support(dev, t[live], lo[live], hi[live], support_drop)
                     for k, v in got_iv.items():
@@ -263,5 +297,27 @@ class Scan:
                         fh.writelines(support_mod.format_support(plan, dev.order, T, iA, ix, ia, ns, iv))
         finally:
             dev.close()
+        if setup is not None:
+            null_T = self._scan_null(setup, device, rank, world, local_rank)
+            if rank == 0:
+                p = null_mod.pvalues(np.where(gap, np.nan, T), null_T)
+                self.null, self.pvalues = null_T, p
+                for line in null_mod.summary(null_T, setup.rep, setup.n_replicates):
+                    print(line)
+                with open(pvalues, 'w') as fh:
+                    fh.writelines(null_mod.format_pvalues(plan, dev.order, T, iA, ix, ia, ns, p))
         if rank == 0:
             print(f'{datetime.now()}. Scan finished.')
+
+    @staticmethod
+    def _scan_null(setup, device, rank, world, local_rank):
+        """CLR of every null row (rank 0; None elsewhere): one segmented load, one scan or one sharded scan."""
+        ndev = DeviceScan.from_problem(setup.problem, setup.order, device=device)
+        try:
+            if world > 1:
+                got = scan_rows_multi_gpu(ndev, setup.t, setup.lo, setup.hi, rank, world, local_rank)
+                end_group()
+                return None if got is None else got[0]
+            return ndev.run(setup.t, setup.lo, setup.hi)[0]
+        finally:
+            ndev.close()

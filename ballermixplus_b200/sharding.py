@@ -10,10 +10,16 @@ count, because centres near sequence ends and in sparse regions are cheaper.
 import numpy as np
 
 
-def centre_costs(genpos, t, lo, hi, A):
-    """Sites a centre touches, summed over the A grid (the kernel's work per centre / n_xa)."""
+def centre_costs(genpos, t, lo, hi, A, seg_start=None):
+    """Sites a centre touches, summed over the A grid (the kernel's work per centre / n_xa).
+
+    ``seg_start``: first site of each segment of a segmented problem (blmx_load_segmented), inside which
+    genpos is non-decreasing.  A window inside one segment is then cut at alpha reach within that segment, as
+    the kernel cuts it; a window across a boundary is charged whole."""
     genpos = np.asarray(genpos)
     t = np.asarray(t, dtype=np.float64)
+    if seg_start is not None and len(seg_start) > 1:
+        return _segmented_costs(genpos, t, lo, hi, A, np.asarray(seg_start, dtype=np.int64))
     cost = np.zeros(len(t), dtype=np.float64)
     sorted_ok = len(genpos) < 2 or bool(np.all(np.diff(genpos) >= 0))
     for a in np.asarray(A, dtype=np.float64):
@@ -25,6 +31,34 @@ def centre_costs(genpos, t, lo, hi, A):
             l, h = np.asarray(lo), np.asarray(hi)
         cost += np.maximum(h - l + 1, 0)
     return cost + 1.0          # never zero: every centre costs a launch slot
+
+
+def _segmented_costs(genpos, t, lo, hi, A, seg_start):
+    n = len(genpos)
+    ends = np.append(seg_start[1:], n)
+    # the library treats the whole problem as unsorted when any segment is (blmx_load_segmented)
+    d = np.diff(genpos) >= 0
+    d[seg_start[1:] - 1] = True
+    sorted_ok = bool(np.all(d)) and not np.any(np.isnan(genpos[seg_start]))
+    L = np.maximum(np.asarray(lo, dtype=np.int64), 0)
+    H = np.minimum(np.asarray(hi, dtype=np.int64), n - 1)
+    seg = np.clip(np.searchsorted(seg_start, L, 'right') - 1, 0, len(seg_start) - 1)
+    inside = sorted_ok & (L <= H) & (H < ends[seg])
+    idx = np.flatnonzero(inside)
+    idx = idx[np.argsort(seg[idx], kind='stable')]          # the centres of each segment, together
+    segs, first = np.unique(seg[idx], return_index=True)
+    groups = [(s, idx[b:e]) for s, b, e in zip(segs, first, np.append(first[1:], len(idx)))]
+    cost = np.zeros(len(t), dtype=np.float64)
+    for a in np.asarray(A, dtype=np.float64):
+        l, h = L.copy(), H.copy()
+        if a > 0:
+            r = 18.420680743952367 / a
+            for s, m in groups:
+                b, e = seg_start[s], ends[s]
+                l[m] = np.maximum(np.searchsorted(genpos[b:e], t[m] - r, 'left') + b, L[m])
+                h[m] = np.minimum(np.searchsorted(genpos[b:e], t[m] + r, 'right') - 1 + b, H[m])
+        cost += np.maximum(h - l + 1, 0)
+    return cost + 1.0
 
 
 def partition(costs, world):
@@ -80,7 +114,7 @@ def gather_rows(rows, counts, rank, world, dist, torch, dst=0):
     return None
 
 
-def scan_sharded(genpos, A, t, lo, hi, rank, world, scan_fn, dist, torch):
+def scan_sharded(genpos, A, t, lo, hi, rank, world, scan_fn, dist, torch, seg_start=None):
     """Scan one sequence's centres on `world` ranks and gather the rows on rank 0.
 
     `scan_fn(t, lo, hi)` scans a contiguous slice of the centre list on this rank's device and
@@ -88,8 +122,9 @@ def scan_sharded(genpos, A, t, lo, hi, rank, world, scan_fn, dist, torch):
     product passes ``DeviceScan.run_device``, i.e. ``blmx_scan_device`` on torch's current stream, so the
     rows never leave the GPU before the gather; CPU tests pass the oracle).
     Returns the five gathered tensors on rank 0 (in centre order) and None elsewhere.
+    ``seg_start``: the segment starts of a segmented problem, for the costs.
     """
-    costs = centre_costs(genpos, t, lo, hi, A)
+    costs = centre_costs(genpos, t, lo, hi, A, seg_start)
     parts = partition(costs, world)
     counts = [e - b for b, e in parts]
     b, e = parts[rank]

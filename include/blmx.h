@@ -99,6 +99,18 @@ int blmx_destroy(blmx_handle *h);
 int blmx_load(blmx_handle *h, const blmx_problem *p);
 
 /*
+ * blmx_load for a problem made of several sequences laid end to end (for example the neutral replicates of
+ * an empirical null).  Segment s is the site range [seg_start[s], seg_start[s+1]) (the last one ends at
+ * n_sites); seg_start[0] == 0, the starts strictly increase and each is < n_sites, n_segments >= 1, else
+ * BLMX_ERR_ARG.  Segments only say where genpos is non-decreasing: the sites a centre uses are exactly those
+ * of blmx_scan's definition.  A window [lo, hi] inside one segment gets the fast paths of a sorted sequence
+ * (distance cut, far field, pruning); a window that crosses a segment boundary is legal and exact, and is
+ * evaluated like a window of unsorted input.  If any segment is not non-decreasing (or holds NaN), the whole
+ * problem is treated as unsorted, as blmx_load treats such input.  n_segments == 1 is blmx_load.
+ */
+int blmx_load_segmented(blmx_handle *h, const blmx_problem *p, int64_t n_segments, const int64_t *seg_start);
+
+/*
  * Scan a batch of centres; HOST buffers in and out (H2D of the centre arrays,
  * kernels, D2H of the results, synchronous).  For centre j the sites used are
  * those with lo[j] <= i <= hi[j] (window_indice, inclusive), exp(-A*|genpos[i]-t[j]|)
@@ -170,7 +182,8 @@ int blmx_scan_oneshot(int device, const blmx_problem *p, int64_t n_centres, cons
  *                have T <= 0 at every grid point and skip their exact evaluation (their candidate is the
  *                all-zero one whatever their exact T, so the rows do not change); 0 = evaluate every item.
  *                Only the default scan prunes: not with report_all, surfaces or profiles, group 1,
- *                farfield 0, unsorted positions or class rows with inf/nan
+ *                farfield 0, unsorted positions or class rows with inf/nan (nor items whose window crosses
+ *                a segment boundary of blmx_load_segmented)
  */
 int blmx_set_option(blmx_handle *h, const char *name, int64_t value);
 
