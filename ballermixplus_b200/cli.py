@@ -3,7 +3,8 @@
 Same flags, defaults, precedence and console messages as the reference's ``main``
 (/root/reference/BalLeRMix+_v1.py:715-802); one extra flag, ``--device``, picks the
 GPU, ``--support`` / ``--supportDrop`` write support intervals of A_hat, x_hat and s_hat (support.py), and
-``--null`` / ``--pvalues`` write empirical p-values from scans of neutral replicates (null.py).
+``--null`` / ``--pvalues`` write empirical p-values from scans of neutral replicates (null.py), and ``--refine``
+/ ``--refineSteps`` write the rows again at the best point of a finer grid around each maximum (refine.py).
 Differences, all on paths where the reference raises (SURVEY.md appendix A.2,
 DESIGN.md "flags without a reference behaviour"): ``--rangeA``, ``--findPos`` and
 ``--minCount`` with ``--noFreq`` work here.
@@ -18,6 +19,7 @@ from .helpers import getConfig, getSpect
 from .inputs import InputData
 from .neutral import NeutralSFS
 from .null import read_list
+from .refine import DEFAULT_STEPS, MAX_STEPS, check_steps
 from .scan import Scan
 from .selection import NormalizedBetaBinom
 from .support import DEFAULT_DROP, check_drop
@@ -83,7 +85,23 @@ def build_parser():
                         'give a region-level threshold). Needs --pvalues.')
     p.add_argument('--pvalues', dest='pvalues', default=None,
                    help='With --null: write FILE with physPos, genPos, CLR and p_value per output row.')
+    p.add_argument('--refine', dest='refine', default=None,
+                   help='Also write FILE, in the output\'s format: every row with CLR > 0 whose best point on a grid '
+                        '--refineSteps times finer (geometric steps for A and alpha, arithmetic for x), inside a box '
+                        'of one coarse step either side of the row\'s maximum, beats its CLR takes that point; every '
+                        'other row is copied. A refined CLR is a maximum over more points, so it is biased upward '
+                        'relative to the coarse CLR and must not be compared with --null CLRs; it is still a grid '
+                        'maximum, not a continuous MLE. One GPU only (not under torchrun).')
+    p.add_argument('--refineSteps', dest='refineSteps', type=_steps, default=DEFAULT_STEPS,
+                   help=f'Fine points per coarse step of --refine, 1 to {MAX_STEPS}. Default {DEFAULT_STEPS}.')
     return p
+
+
+def _steps(text):
+    try:
+        return check_steps(text)
+    except ValueError as exc:
+        raise argparse.ArgumentTypeError(str(exc)) from None
 
 
 def _drop(text):
@@ -104,6 +122,8 @@ def main(argv=None):
     opt = parser.parse_args(argv)
     if opt.support is not None and int(os.environ.get('WORLD_SIZE', '1')) > 1:
         parser.error('--support runs on one GPU; launch without torchrun (WORLD_SIZE > 1)')
+    if opt.refine is not None and int(os.environ.get('WORLD_SIZE', '1')) > 1:
+        parser.error('--refine runs on one GPU; launch without torchrun (WORLD_SIZE > 1)')
     if (opt.null is None) != (opt.pvalues is None):
         parser.error('--null and --pvalues must be given together')
     if opt.null is not None:
@@ -142,7 +162,8 @@ def main(argv=None):
     print('\n%s. Start computing likelihood raito...' % (datetime.now()))
     Scan(data, Neutral, Sel_Probs, grid, opt.outfile, fixSize=opt.size, r=opt.w, s=opt.step,
          phys=opt.phys, noCenter=opt.noCenter, device=opt.device, support=opt.support,
-         support_drop=opt.supportDrop, null=opt.null, pvalues=opt.pvalues)
+         support_drop=opt.supportDrop, null=opt.null, pvalues=opt.pvalues, refine=opt.refine,
+         refine_steps=opt.refineSteps)
     print(f'\n{datetime.now()}. Pipeline finished.')
 
 

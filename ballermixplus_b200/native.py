@@ -18,7 +18,7 @@ ABI_SYMBOLS = (
     'blmx_load', 'blmx_scan', 'blmx_scan_device', 'blmx_scan_oneshot', 'blmx_set_option',
     'blmx_last_counters', 'blmx_last_counters6', 'blmx_last_counters8', 'blmx_last_counters9', 'blmx_problem_info',
     'blmx_last_kernel_ms', 'blmx_measure_fp64_peak', 'blmx_scan_profile', 'blmx_scan_surface',
-    'blmx_load_segmented',
+    'blmx_load_segmented', 'blmx_load_refine', 'blmx_refine',
 )
 
 
@@ -67,6 +67,10 @@ def lib():
                                        C.POINTER(Result), C.c_void_p]
         L.blmx_scan_oneshot.argtypes = [C.c_int, C.POINTER(Problem), C.c_int64, C.c_void_p,
                                         C.c_void_p, C.c_void_p, C.POINTER(Result)]
+        L.blmx_load_refine.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int64,
+                                       C.c_void_p, C.c_void_p]
+        L.blmx_refine.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                  C.POINTER(Result)]
         L.blmx_set_option.argtypes = [C.c_void_p, C.c_char_p, C.c_int64]
         L.blmx_last_counters.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64),
                                          C.POINTER(C.c_uint64)]
@@ -210,6 +214,33 @@ class Scanner:
         nsA = np.zeros((n, n_A), np.int32)
         _check(lib().blmx_scan_surface(self._h, n, _ptr(t), _ptr(lo), _ptr(hi), _ptr(S), _ptr(nsA)))
         return S, nsA
+
+    def load_refine(self, fA, n_fx, n_fa, row_of, SP):
+        """Fine tables of blmx_load_refine: fine A values, the fine (x, a) axis lengths, row_of [n_fx * n_fa]
+        (row of SP or -1) and SP [n_rows, n_classes]."""
+        fA = np.ascontiguousarray(fA, dtype=np.float64)
+        row_of = np.ascontiguousarray(row_of, dtype=np.int32)
+        SP = np.ascontiguousarray(SP, dtype=np.float64)
+        if row_of.shape != (int(n_fx) * int(n_fa),):
+            raise ValueError('row_of must have n_fx * n_fa entries')
+        n_rows = SP.shape[0] if SP.ndim == 2 else 0
+        _check(lib().blmx_load_refine(self._h, len(fA), _ptr(fA), int(n_fx), int(n_fa), n_rows, _ptr(row_of),
+                                      _ptr(SP)))
+        self._refine_tables = (fA, row_of, SP)
+
+    def refine(self, t, lo, hi, box):
+        """Box maxima of the fine grid (blmx_refine); box is int [n, 6] -> (T, fA, fx, fa, nsites), fine
+        indices."""
+        t, lo, hi = self._centres(t, lo, hi)
+        box = np.ascontiguousarray(box, dtype=np.int32)
+        n = len(t)
+        if box.shape != (n, 6):
+            raise ValueError('box must be [n, 6]')
+        T = np.full(n, -np.inf)
+        fA, fx, fa, ns = (np.full(n, -1, np.int32) for _ in range(4))
+        res = Result(_ptr(T), _ptr(fA), _ptr(fx), _ptr(fa), _ptr(ns))
+        _check(lib().blmx_refine(self._h, n, _ptr(t), _ptr(lo), _ptr(hi), _ptr(box), C.byref(res)))
+        return T, fA, fx, fa, ns
 
     def scan_device(self, n, d_t, d_lo, d_hi, d_T, d_iA, d_ix, d_ia, d_ns, stream=0):
         """Raw DEVICE pointers (ints) in and out, asynchronous on `stream`."""

@@ -11,7 +11,7 @@ from datetime import datetime
 
 import numpy as np
 
-from . import fastio, null as null_mod, support as support_mod, windows
+from . import fastio, null as null_mod, refine as refine_mod, support as support_mod, windows
 from .native import Scanner
 from .problem import build_problem
 
@@ -49,6 +49,14 @@ class DeviceScan:
     def surface(self, t, lo, hi):
         """The whole likelihood surface of a few centres -> (S [n, n_A, n_x, n_a], nsA [n, n_A])."""
         return self.scanner.scan_surface(t, lo, hi)
+
+    def load_refine(self, fA, n_fx, n_fa, row_of, SP):
+        """Fine tables for ``refine`` (refine.py builds them)."""
+        self.scanner.load_refine(fA, n_fx, n_fa, row_of, SP)
+
+    def refine(self, t, lo, hi, box):
+        """Box maxima of the fine grid -> (T, fA, fx, fa, nsites), fine indices (refine.py)."""
+        return self.scanner.refine(t, lo, hi, box)
 
     def run_device(self, t, lo, hi, torch, device):
         """Same scan with the centres uploaded once and the results LEFT ON THE DEVICE as torch tensors
@@ -236,16 +244,25 @@ class Scan:
 
     ``null`` (a replicate list) and ``pvalues`` (a path), given together: also scan the neutral replicates the
     list names with the same flags and tables, as one segmented problem, and write, per row of ``outfile``,
-    its empirical p-value against the pooled null CLRs (null.py).  ``outfile`` is the same either way."""
+    its empirical p-value against the pooled null CLRs (null.py).  ``outfile`` is the same either way.
+
+    ``refine`` (a path): also write ``outfile`` again with every row with T > 0 replaced by the best point of a
+    grid ``refine_steps`` times finer inside a box around its maximum, where that point beats the row's CLR
+    (refine.py).  One GPU only.  ``outfile``, the support and the p-value files stay on the coarse grid."""
 
     def __init__(self, InputData, NeutralSFS, NormalizedBetaBinom, Grids, outfile, fixSize=False,
                  r=0, s=1, phys=False, noCenter=False, device=0, support=None,
-                 support_drop=support_mod.DEFAULT_DROP, null=None, pvalues=None):
+                 support_drop=support_mod.DEFAULT_DROP, null=None, pvalues=None, refine=None,
+                 refine_steps=refine_mod.DEFAULT_STEPS):
         rank, world, local_rank = _world()
         if support is not None:
             support_drop = support_mod.check_drop(support_drop)
             if world > 1:
                 raise ValueError('--support runs on one GPU: launch without torchrun (WORLD_SIZE > 1)')
+        if refine is not None:
+            refine_steps = refine_mod.check_steps(refine_steps)
+            if world > 1:
+                raise ValueError('--refine runs on one GPU: launch without torchrun (WORLD_SIZE > 1)')
         if (null is None) != (pvalues is None):
             raise ValueError('--null and --pvalues go together')
         plan = windows.make_plan(InputData, fixSize=fixSize, r=r, s=s, phys=phys, noCenter=noCenter)
@@ -260,6 +277,9 @@ class Scan:
                     pass
             if pvalues is not None:
                 with open(pvalues, 'w'):
+                    pass
+            if refine is not None:
+                with open(refine, 'w'):
                     pass
         setup = None
         if null is not None:
@@ -295,6 +315,8 @@ class Scan:
                     with open(support, 'w') as fh:
                         fh.write(support_mod.SUPPORT_HEADER)
                         fh.writelines(support_mod.format_support(plan, dev.order, T, iA, ix, ia, ns, iv))
+                if refine is not None:
+                    self._refine(dev, NeutralSFS, NormalizedBetaBinom, refine_steps, refine, plan, t, lo, hi)
         finally:
             dev.close()
         if setup is not None:
@@ -308,6 +330,19 @@ class Scan:
                     fh.writelines(null_mod.format_pvalues(plan, dev.order, T, iA, ix, ia, ns, p))
         if rank == 0:
             print(f'{datetime.now()}. Scan finished.')
+
+    def _refine(self, dev, neutral, sel, K, path, plan, t, lo, hi):
+        """Refine the rows of ``self.results`` on ``dev`` and write the refine file."""
+        T, iA, ix, ia, ns = self.results
+        grid, rows = refine_mod.refine_rows(dev, neutral, sel, K, t, lo, hi, iA, ix, ia)
+        move = refine_mod.moved(grid, T, iA, ix, ia, rows)
+        self.refined, self.refine_grid, self.moved = rows, grid, move
+        with open(path, 'w') as fh:
+            fh.write(HEADER)
+            fh.writelines(refine_mod.format_refined(plan, format_rows(plan, dev.order, T, iA, ix, ia, ns), grid,
+                                                    rows, move))
+        print(f'refine (K = {grid.K}): {int(move.sum())} of {int((iA >= 0).sum())} rows with T > 0 moved to a '
+              f'finer grid point')
 
     @staticmethod
     def _scan_null(setup, device, rank, world, local_rank):

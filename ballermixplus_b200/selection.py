@@ -85,6 +85,30 @@ class NormalizedBetaBinom:
         """Per-site normalised selection probabilities (reference API, v1:362)."""
         return self.classProbs[(x, a)][self.cls]
 
+    def rows_at(self, pairs):
+        """float64 [len(pairs), C]: the class rows at an explicit list of (x, a) points, with the constructor's
+        arithmetic (one broadcast pmf per sample size and side of the fold), so a point of the scan's grid gets
+        the bits of ``classProbs[(x, a)]``.  The fine grid of refine.py uses it."""
+        out = np.zeros((len(pairs), len(self.class_k)))
+        if not len(pairs):
+            return out
+        avec = np.array([float(a) for _, a in pairs])
+        for n in sorted(set(self.class_n.tolist())):
+            members = np.flatnonzero(self.class_n == n)
+            j = np.arange(n + 1)
+            pmf = []
+            for side in (lambda x: x, lambda x: 1. - x):
+                bvec = np.array([self._get_b(side(x), a) for x, a in pairs], dtype=np.float64)
+                pmf.append(betabinom.pmf(j[None, :], n, avec[:, None], bvec[:, None]))
+            k = self.class_k[members]
+            excl = self._excluded(n)
+            for r in range(len(pairs)):
+                px, pc = pmf[0][r], pmf[1][r]
+                folded = 0.5 * (self._raw_from(px, k, n) + self._raw_from(pc, k, n))
+                base = 1. - np.sum(0.5 * (px[excl] + pc[excl]))
+                out[r, members] = folded / base
+        return out
+
     # -- pieces -----------------------------------------------------------------
     def _raw_from(self, p, k, n):
         """Unfolded probabilities of the classes k from the pmf p[0..n] (v1:375-396)."""

@@ -159,6 +159,30 @@ int blmx_scan_profile(blmx_handle *h, int64_t n_centres, const double *t, const 
 int blmx_scan_surface(blmx_handle *h, int64_t n_centres, const double *t, const int64_t *lo,
                       const int64_t *hi, double *S, int32_t *nsA);
 
+/*
+ * Local grid refinement (DESIGN.md §3.10): the best point of a finer grid inside a box around each centre's
+ * coarse maximum.  The fine grid is given by axes, not by the problem's grid: n_fA fine A values, and n_fx x
+ * n_fa fine (x, a) points of which only those that some box needs have a class row.
+ *
+ * blmx_load_refine loads the fine tables for the problem already on the handle (else BLMX_ERR_STATE):
+ *   fA[i]                 fine A values
+ *   row_of[ix*n_fa + ia]  row of SP for fine point (ix, ia), or -1 where no box may go
+ *   SP[row][c]            NormalizedBetaBinom probabilities * propSizes at that point (as blmx_problem.SP)
+ * R = SP/G is formed with the G of the loaded problem, as blmx_load forms it.  The next blmx_load or
+ * blmx_load_segmented drops the fine tables.
+ *
+ * blmx_refine takes, per centre, the window of blmx_scan and box[j][6] = fA0, fA1, fx0, fx1, fa0, fa1, inclusive
+ * ranges of fine indices.  Every point of every box must have a row, a box may hold at most 17 x 17 (x, a)
+ * points, and no range may be empty or leave its axis (else BLMX_ERR_ARG).  The result, in fine indices, is the
+ * box maximum: visiting order fine A, then fine x, then fine a, strict '>' starting from -inf (NaN never wins),
+ * an A without sites skipped; T = -inf and -1 indices where nothing qualifies.  There is no far field and no
+ * pruning: every site of the window is multiplied in at every point.  HOST buffers, synchronous.
+ */
+int blmx_load_refine(blmx_handle *h, int64_t n_fA, const double *fA, int64_t n_fx, int64_t n_fa, int64_t n_rows,
+                     const int32_t *row_of, const double *SP);
+int blmx_refine(blmx_handle *h, int64_t n_centres, const double *t, const int64_t *lo, const int64_t *hi,
+                const int32_t *box, const blmx_result *out);
+
 /* One-shot form of the seam: create + load + scan + destroy on `device`. */
 int blmx_scan_oneshot(int device, const blmx_problem *p, int64_t n_centres, const double *t,
                       const int64_t *lo, const int64_t *hi, const blmx_result *out);
@@ -196,7 +220,7 @@ int blmx_set_option(blmx_handle *h, const char *name, int64_t value);
  */
 int blmx_last_counters(blmx_handle *h, uint64_t *site_pairs, uint64_t *single_pairs,
                        uint64_t *launches);
-/* All work counters: [0] site_pairs, [1] single_pairs, [2] far-field block visits (one exp and
+/* All work counters (blmx_refine resets them and counts [5] only): [0] site_pairs, [1] single_pairs, [2] far-field block visits (one exp and
  * one DFMA on each of 32 lanes), [3] far-field polynomial terms summed over class visits (one DFMA
  * per term and grid point), [4] site pairs that entered through the far field, [5] index-range
  * violations (always 0; counted only by the -DBLMX_CHECKED build the tests run), [6] of [4], the

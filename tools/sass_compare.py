@@ -5,7 +5,8 @@
 Every scan_kernel<J, GROUP, FAR> of OLD (the kernel before it took the SURF flag) is compared, instruction
 listing for instruction listing (cuobjdump -sass), with scan_kernel<J, GROUP, FAR, SURF = false> of NEW; a
 kernel OLD already has with the SURF flag is compared with the same instantiation in NEW.  Build both with the
-same nvcc flags.  Exit status 1 if any listing differs.
+same nvcc flags.  bound_kernel, which the scan runs before scan_kernel, is compared as well.  Exit status 1 if any
+listing differs.
 """
 import re
 import subprocess
@@ -14,8 +15,8 @@ import sys
 CUDA_BIN = '/usr/local/cuda/bin'
 
 
-def scan_kernels(so):
-    """{'scan_kernel<J, GROUP, FAR[, SURF]>': SASS listing} of a library."""
+def scan_kernels(so, prefix='scan_kernel<'):
+    """{'scan_kernel<J, GROUP, FAR[, SURF]>': SASS listing} of a library (prefix 'bound_kernel(': that kernel)."""
     out = subprocess.run([f'{CUDA_BIN}/cuobjdump', '-sass', so], capture_output=True, text=True, check=True).stdout
     parts = re.split(r'\n\s*Function : (\S+)\n', out)
     names = subprocess.run([f'{CUDA_BIN}/cu++filt'], input='\n'.join(parts[1::2]), capture_output=True, text=True,
@@ -23,8 +24,9 @@ def scan_kernels(so):
     res = {}
     for name, body in zip(names, parts[2::2]):
         name = name.replace('<unnamed>::', '').replace('(int)', '').replace('(bool)', '')
-        if name.startswith('void scan_kernel<'):
-            res[name[len('void '):name.index('>') + 1]] = body
+        name = name[len('void '):] if name.startswith('void ') else name      # templates carry their return type
+        if name.startswith(prefix):
+            res[name[:name.index('>' if prefix.endswith('<') else '(') + 1]] = body
     return res
 
 
@@ -37,7 +39,11 @@ def main():
         same += ok
         print(f'{"identical" if ok else "DIFFERENT"}  {name} -> {twin}  ({len(old[name].splitlines())} lines)')
     print(f'{same}/{len(old)} identical')
-    return 0 if same == len(old) else 1
+    old_b, new_b = scan_kernels(sys.argv[1], 'bound_kernel('), scan_kernels(sys.argv[2], 'bound_kernel(')
+    same_b = sum(old_b[k] == new_b.get(k) for k in old_b)
+    for k in sorted(old_b):
+        print(f'{"identical" if old_b[k] == new_b.get(k) else "DIFFERENT"}  {k}  ({len(old_b[k].splitlines())} lines)')
+    return 0 if same == len(old) and same_b == len(old_b) else 1
 
 
 if __name__ == '__main__':
