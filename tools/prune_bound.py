@@ -18,6 +18,14 @@ Variant 'jensen' (what bound_kernel evaluates, DESIGN.md §3.8): log(1 + alpha D
 sites of a class in one alpha bin give at most n log(1 + abar D); two bins split at alpha* (K unused).  The kernel's
 decision margin (1e-4 of the sum of |terms| plus 1e-5, in log2 units) is applied here too.
 
+Cluster stage (DESIGN.md §3.8): for clusters of K consecutive xa, log2(1 + abar D) is non-decreasing in D, so
+B_cl = sum n log2(1 + abar Dmax) bounds B at every point of the cluster and A_cl = sum n max(|l(Dmax)|, |l(Dmin)|)
+bounds its margin term; a cluster is settled when B_cl + 1e-4 A_cl + 1e-5 < 0.  For each K the tool reports the
+fraction of grid points settled that way and a model of the lg2 evaluations per item: 2 per (class, bin, cluster),
+then K per (class, bin) for each open cluster, visited in order of decreasing B_cl until one has a point that
+fails; against 128 per (class, bin) for each 128-point pass of the point-by-point evaluation, which stops after
+the first pass with a failing point.
+
 Usage: python tools/prune_bound.py [--sites 1000000] [--centres 30] [--out profiles/r4_prune_bound.json]
 """
 import argparse
@@ -78,6 +86,61 @@ def bound_per_grid_point(alpha, cls, D, logR, K, a_star, variant):
     return (tail + nb).sum(-1)
 
 
+CLUSTERS = (4, 8, 16, 32)
+
+
+def jensen_terms(alpha, cls, C, a_star=0.5):
+    """(n, abar) of every (class, bin) with sites: the statistics bound_kernel keeps."""
+    near = alpha >= a_star
+    ns, ab = [], []
+    for m in (~near, near):
+        cnt = np.bincount(cls[m], minlength=C).astype(np.float64)
+        s1 = np.bincount(cls[m], weights=alpha[m], minlength=C)
+        k = cnt > 0
+        ns.append(cnt[k]); ab.append(s1[k] / cnt[k])
+    return np.concatenate(ns), np.concatenate(ab), np.concatenate([np.nonzero(np.bincount(
+        cls[m], minlength=C))[0] for m in (~near, near)])
+
+
+def cluster_stats(D, K):
+    """Dmax, Dmin [n_cl, C] over clusters of K consecutive grid points, and the points of each cluster."""
+    n_xa = D.shape[0]
+    n_cl = (n_xa + K - 1) // K
+    Dmax = np.stack([D[j * K:(j + 1) * K].max(0) for j in range(n_cl)])
+    Dmin = np.stack([D[j * K:(j + 1) * K].min(0) for j in range(n_cl)])
+    pts = np.array([min(K, n_xa - j * K) for j in range(n_cl)])
+    return Dmax, Dmin, pts
+
+
+def cluster_model(n, abar, c_of, D, clusters):
+    """Settled points and modelled lg2 count for one item, for each cluster shape; plus the point-by-point count."""
+    with np.errstate(divide='ignore', invalid='ignore'):
+        lp = n * np.log2(1.0 + D[:, c_of] * abar)                            # [n_xa, terms]
+    per_pt = lp.sum(-1) + 1e-4 * np.abs(lp).sum(-1) + 1e-5
+    fail_pt = ~(per_pt < 0)
+    nt = len(n)
+    n_xa = D.shape[0]
+    passes = (n_xa + 127) // 128
+    first_fail_pass = next((k for k in range(passes) if fail_pt[k * 128:(k + 1) * 128].any()), passes - 1)
+    res = {'points_lg2': 128 * nt * (first_fail_pass + 1)}
+    for K, (Dmax, Dmin, pts) in clusters.items():
+        with np.errstate(divide='ignore', invalid='ignore'):
+            lmax = n * np.log2(1.0 + Dmax[:, c_of] * abar)
+            lmin = n * np.log2(1.0 + Dmin[:, c_of] * abar)
+        Bc = lmax.sum(-1)
+        Ac = np.maximum(np.abs(lmax), np.abs(lmin)).sum(-1)
+        settled = Bc + 1e-4 * Ac + 1e-5 < 0
+        lg2 = 2 * nt * len(Bc)
+        for j in np.argsort(-np.where(np.isnan(Bc), np.inf, Bc), kind='stable'):
+            if settled[j]:
+                continue
+            lg2 += K * nt
+            if fail_pt[j * K:(j + 1) * K].any():
+                break
+        res[K] = {'settled_points': int(pts[settled].sum()), 'lg2': int(lg2)}
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--sites', type=int, default=1_000_000)
@@ -102,6 +165,8 @@ def main():
     iAs = np.arange(0, len(p.A), opt.every_a)
     configs = [(v, K, a) for v in ('issue', 'best') for K in (3, 5) for a in (0.5, 0.9)] + [('jensen', 0, 0.5)]
     rec = {c: {'proved': 0, 'proved_pairs': 0, 'violations': 0, 'slack': []} for c in configs}
+    clusters = {K: cluster_stats(D, K) for K in CLUSTERS}
+    crec = {'points_lg2': 0, **{K: {'settled_points': 0, 'lg2': 0} for K in CLUSTERS}}
     items = pos_items = 0
     pairs_total = 0
     exact_max = []
@@ -118,6 +183,11 @@ def main():
             pos_items += Tex > 0
             pairs_total += len(alpha)
             exact_max.append(Tex)
+            cm = cluster_model(*jensen_terms(alpha, cls, D.shape[1]), D, clusters)
+            crec['points_lg2'] += cm['points_lg2']
+            for K in CLUSTERS:
+                for k in ('settled_points', 'lg2'):
+                    crec[K][k] += cm[K][k]
             for c in configs:
                 b = 2.0 * bound_per_grid_point(alpha, cls, D, logR, c[1], c[2], c[0])
                 bmax = float(np.max(b))
@@ -140,6 +210,9 @@ def main():
                               'frac_site_pairs_proved': r['proved_pairs'] / pairs_total,
                               'bound_below_exact': r['violations'],
                               'slack_bound_minus_exact_quantiles': np.quantile(s, [0, .1, .5, .9, 1]).tolist()})
+    out['clusters'] = {'grid_points': int(D.shape[0]), 'lg2_per_item_point_by_point': crec['points_lg2'] / items,
+                       'shapes': [{'K': K, 'frac_points_settled': crec[K]['settled_points'] / (items * D.shape[0]),
+                                   'lg2_per_item': crec[K]['lg2'] / items} for K in CLUSTERS]}
     out['seconds'] = time.time() - t0
     line = json.dumps(out, indent=1)
     print(line)
