@@ -3,8 +3,9 @@
 Same flags, defaults, precedence and console messages as the reference's ``main``
 (/root/reference/BalLeRMix+_v1.py:715-802); one extra flag, ``--device``, picks the
 GPU, ``--support`` / ``--supportDrop`` write support intervals of A_hat, x_hat and s_hat (support.py), and
-``--null`` / ``--pvalues`` write empirical p-values from scans of neutral replicates (null.py), and ``--refine``
-/ ``--refineSteps`` write the rows again at the best point of a finer grid around each maximum (refine.py).
+``--null`` / ``--pvalues`` write empirical p-values from scans of neutral replicates (null.py), ``--refine``
+/ ``--refineSteps`` write the rows again at the best point of a finer grid around each maximum (refine.py), and
+``--inputList`` scans one input per chromosome in one run (scan.GenomeScan).
 Differences, all on paths where the reference raises (SURVEY.md appendix A.2,
 DESIGN.md "flags without a reference behaviour"): ``--rangeA``, ``--findPos`` and
 ``--minCount`` with ``--noFreq`` work here.
@@ -20,7 +21,7 @@ from .inputs import InputData
 from .neutral import NeutralSFS
 from .null import read_list
 from .refine import DEFAULT_STEPS, MAX_STEPS, check_steps
-from .scan import Scan
+from .scan import GenomeScan, Scan, input_list, list_outputs
 from .selection import NormalizedBetaBinom
 from .support import DEFAULT_DROP, check_drop
 
@@ -92,6 +93,13 @@ def build_parser():
                         'other row is copied. A refined CLR is a maximum over more points, so it is biased upward '
                         'relative to the coarse CLR and must not be compared with --null CLRs; it is still a grid '
                         'maximum, not a continuous MLE. One GPU only (not under torchrun).')
+    p.add_argument('--inputList', dest='inputList', action='store_true', default=False,
+                   help='Scan a genome in one run: -i names a text file listing one input per line (one per '
+                        'chromosome; relative to the list, blank and # lines skipped), and -o, --support, '
+                        '--pvalues and --refine name existing directories. Input chr7.txt writes DIR/chr7.txt, '
+                        'the file a run on chr7.txt alone with the same flags writes. The --null replicates are '
+                        'scanned once for all inputs. Under torchrun the whole genome is sharded over the GPUs. '
+                        'With --getSpect or --getConfig: the helper file of all listed inputs together.')
     p.add_argument('--refineSteps', dest='refineSteps', type=_steps, default=DEFAULT_STEPS,
                    help=f'Fine points per coarse step of --refine, 1 to {MAX_STEPS}. Default {DEFAULT_STEPS}.')
     return p
@@ -132,16 +140,23 @@ def main(argv=None):
         except (OSError, ValueError) as exc:
             parser.error(str(exc))
 
+    inputs = opt.infile
+    if opt.inputList:
+        inputs = _check_list_mode(parser, opt)
+
     if opt.getSpec:
         print('You\'ve chosen to generate site frequency spectrum...')
         print('Concatenated input: %s \nSpectrum file: %s' % (opt.infile, opt.spectfile))
-        getSpect(opt.infile, opt.spectfile, opt.MAF, opt.nosub)
+        getSpect(inputs, opt.spectfile, opt.MAF, opt.nosub)
         sys.exit()
     elif opt.getConfig:
         print('You\'ve chosen to generate the substitution-polymorphism configuration...')
         print('Concatenated input: %s \nConfiguration file: %s' % (opt.infile, opt.spectfile))
-        getConfig(opt.infile, opt.spectfile)
+        getConfig(inputs, opt.spectfile)
         sys.exit()
+    if opt.inputList:
+        _main_list(opt, inputs)
+        return
 
     print(f'\n{datetime.now()}. Reading input from {opt.infile}')
     data = InputData(opt.infile, opt.nofreq, opt.MAF, opt.nosub, opt.minCount, phys=opt.phys,
@@ -164,6 +179,50 @@ def main(argv=None):
          phys=opt.phys, noCenter=opt.noCenter, device=opt.device, support=opt.support,
          support_drop=opt.supportDrop, null=opt.null, pvalues=opt.pvalues, refine=opt.refine,
          refine_steps=opt.refineSteps)
+    print(f'\n{datetime.now()}. Pipeline finished.')
+
+
+def _check_list_mode(parser, opt):
+    """``--inputList``: the inputs the list names; a bad list or output directory fails before any input is
+    read."""
+    try:
+        inputs = input_list(opt.infile)
+    except (OSError, ValueError) as exc:
+        parser.error(str(exc))
+    if opt.getSpec or opt.getConfig:
+        return inputs
+    if opt.outfile is None:
+        parser.error('--inputList needs -o DIR')
+    for flag, d in (('-o', opt.outfile), ('--support', opt.support), ('--pvalues', opt.pvalues),
+                    ('--refine', opt.refine)):
+        if d is not None and not os.path.isdir(d):
+            parser.error(f'--inputList: {flag} {d} is not an existing directory')
+    try:
+        list_outputs(inputs, out=opt.outfile, support=opt.support, pvalues=opt.pvalues, refine=opt.refine)
+    except ValueError as exc:
+        parser.error(str(exc))
+    return inputs
+
+
+def _main_list(opt, inputs):
+    """One run over every listed input (scan.GenomeScan), each read and tabulated as the one-input run reads it."""
+    print(f'\n{datetime.now()}. {len(inputs)} inputs listed in {opt.infile}')
+    Neutral = NeutralSFS(opt.spectfile, opt.nofreq, opt.MAF, opt.nosub)
+    grid = Grids(opt.x, opt.abeta, opt.bal, opt.pos, opt.seqA, opt.listA)
+    print('\nOptimizing over x= ' + ', '.join(['%g' % (x) for x in grid.x]))
+    print('\n \t alpha= ' + ', '.join([str(a) for a in grid.abeta]))
+    print('\n \t A= ' + ', '.join([str(A) for A in grid.A]))
+
+    def read(path):
+        print(f'\n{datetime.now()}. Reading input from {path}')
+        data = InputData(path, opt.nofreq, opt.MAF, opt.nosub, opt.minCount, phys=opt.phys, Rrate=opt.Rrate)
+        Neutral.get_neut_probs(data)
+        return data, NormalizedBetaBinom(data, grid, opt.nofreq, opt.MAF, opt.nosub)
+
+    print('\n%s. Start computing likelihood raito...' % (datetime.now()))
+    GenomeScan(inputs, read, Neutral, grid, opt.outfile, fixSize=opt.size, r=opt.w, s=opt.step, phys=opt.phys,
+               noCenter=opt.noCenter, device=opt.device, support=opt.support, support_drop=opt.supportDrop,
+               null=opt.null, pvalues=opt.pvalues, refine=opt.refine, refine_steps=opt.refineSteps)
     print(f'\n{datetime.now()}. Pipeline finished.')
 
 

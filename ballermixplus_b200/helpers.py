@@ -13,7 +13,11 @@ Rules kept:
     once; note for --MAF this is x == 0); rows sorted by (x, n).
   getConfig (v1:645-664): x == 0 rows are reported and skipped; per n the pair
     [#substitutions (x == n), #polymorphisms]; rows sorted by n.
+
+``infile`` may also be a list of paths (``--inputList``): the helper file is then the one the concatenation of
+the inputs (in list order, first header kept) gives, so a genome-wide spectrum needs no hand-made file.
 """
+import os
 import sys
 
 import numpy as np
@@ -22,6 +26,12 @@ from . import fastio
 
 
 def _read_xn(infile):
+    """(x, n) of every site of `infile`, or, for a list of paths, of the inputs laid end to end in list order:
+    the sites of their concatenation with only the first file's header kept (``--inputList``)."""
+    if not isinstance(infile, (str, bytes, os.PathLike)):
+        parts = [_read_xn(p) for p in infile]
+        return (np.concatenate([x for x, _ in parts]).astype(np.int64),
+                np.concatenate([n for _, n in parts]).astype(np.int64))
     fast = fastio.read_sites(infile, True, 1.0, strict_columns=True)     # C++ reader; None -> the loop below
     if fast is not None:
         return fast[2], fast[3]

@@ -36,12 +36,13 @@ PVALUE_HEADER = 'physPos\tgenPos\tCLR\tp_value\n'
 QUANTILES = (0.95, 0.99, 0.999)
 
 
-def read_list(path):
+def read_list(path, flag='--null', item='replicate'):
     """Replicate input files named by the list `path`, one per line; relative paths are taken from the list's
     directory, blank lines and lines starting with '#' are skipped.  A missing or empty list, or a missing
-    replicate, raises before anything is read."""
+    replicate, raises before anything is read.  `flag` and `item` name the option and what it lists in the
+    messages (``--inputList`` reads its inputs with the same rules)."""
     if not os.path.isfile(path):
-        raise FileNotFoundError(f'--null: replicate list {path} not found')
+        raise FileNotFoundError(f'{flag}: {item} list {path} not found')
     base = os.path.dirname(os.path.abspath(path))
     out = []
     with open(path) as fh:
@@ -51,10 +52,10 @@ def read_list(path):
                 continue
             full = name if os.path.isabs(name) else os.path.join(base, name)
             if not os.path.isfile(full):
-                raise FileNotFoundError(f'--null: replicate {full} (listed in {path}) not found')
+                raise FileNotFoundError(f'{flag}: {item} {full} (listed in {path}) not found')
             out.append(full)
     if not out:
-        raise ValueError(f'--null: replicate list {path} names no replicate')
+        raise ValueError(f'{flag}: {item} list {path} names no {item}')
     return out
 
 

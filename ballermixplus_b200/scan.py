@@ -4,16 +4,18 @@
 (/root/reference/BalLeRMix+_v1.py:436-507 and :510-640); the work is done by the
 CUDA library behind include/blmx.h.  ``Scan`` plans all centres of the run first
 (windows.py), sends them to the GPU in one ``blmx_scan`` call and then writes the
-rows with the reference's f-string formatting.
+rows with the reference's f-string formatting.  ``GenomeScan`` runs ``Scan``'s work over one input per
+chromosome (``--inputList``).
 """
 import os
+import time
 from datetime import datetime
 
 import numpy as np
 
 from . import fastio, null as null_mod, refine as refine_mod, support as support_mod, windows
 from .native import Scanner
-from .problem import build_problem
+from .problem import GridOrder, build_problem
 
 HEADER = 'physPos\tgenPos\tCLR\tx_hat\ts_hat\tA_hat\tnSites\n'
 
@@ -167,6 +169,16 @@ def scan_rows_multi_gpu(dev, t, lo, hi, rank, world, local_rank, keep_group=Fals
     share one device (tests on a one-GPU box) the gather runs over gloo on host tensors.  Returns the five
     result arrays on rank 0 and None elsewhere.  ``keep_group``: leave the process group this call starts
     running for a later scan (``end_group`` ends it)."""
+    seq = (dev.problem.genpos, dev.problem.A, t, lo, hi, getattr(dev.problem, 'seg_start', None))
+    return scan_seqs_multi_gpu([seq], lambda i: dev, dev.scanner.device, rank, world, keep_group=keep_group)
+
+
+def scan_seqs_multi_gpu(seqs, open_dev, device, rank, world, keep_group=False, release=False):
+    """``scan_rows_multi_gpu`` over several sequences (sharding.scan_sharded_seqs): the centres of all of them are
+    cut into cost-balanced ranges, and a rank scans only the sequences its range touches, on the DeviceScan
+    ``open_dev(i)`` gives for sequence i.  ``seqs``: one (genpos, A, t, lo, hi, seg_start) per sequence.
+    ``release``: close each DeviceScan once its rows are computed, so that one sequence at a time is resident.
+    Returns the five result arrays of the concatenated centre list on rank 0 and None elsewhere."""
     import torch
     import torch.distributed as dist
     from . import sharding
@@ -176,25 +188,30 @@ def scan_rows_multi_gpu(dev, t, lo, hi, rank, world, local_rank, keep_group=Fals
         os.environ.setdefault('MASTER_ADDR', '127.0.0.1')
         os.environ.setdefault('MASTER_PORT', '29500')
         if own_gpu:
-            torch.cuda.set_device(dev.scanner.device)
+            torch.cuda.set_device(device)
             dist.init_process_group('nccl', rank=rank, world_size=world,
-                                    device_id=torch.device('cuda', dev.scanner.device))
+                                    device_id=torch.device('cuda', device))
         else:
             dist.init_process_group('gloo', rank=rank, world_size=world)
 
-    if own_gpu:
-        where = torch.device('cuda', dev.scanner.device)
+    where = torch.device('cuda', device) if own_gpu else torch.device('cpu')
 
-        def scan_fn(ts, los, his):
-            return dev.run_device(ts, los, his, torch, where)
-    else:
-        def scan_fn(ts, los, his):
+    def scan_fn(i, ts, los, his):
+        dev = open_dev(i)
+        try:
+            if own_gpu:
+                got = dev.run_device(ts, los, his, torch, where)
+                if release:             # the rows stay on the device; the handle may go once they are written
+                    torch.cuda.current_stream(where).synchronize()
+                return got
             return tuple(torch.from_numpy(np.ascontiguousarray(a)) for a in dev.run(ts, los, his))
+        finally:
+            if release:
+                dev.close()
 
     ok = False
     try:
-        got = sharding.scan_sharded(dev.problem.genpos, dev.problem.A, t, lo, hi, rank, world, scan_fn, dist, torch,
-                                    seg_start=getattr(dev.problem, 'seg_start', None))
+        got = sharding.scan_sharded_seqs(seqs, rank, world, scan_fn, dist, torch, device=where)
         ok = True
         return None if got is None else tuple(a.cpu().numpy() for a in got)
     finally:
@@ -232,6 +249,83 @@ def scan_with_support(dev, t, lo, hi, q):
     return tuple(rows), iv
 
 
+INTERVAL_KEYS = ('A_lo', 'A_hi', 'x_lo', 'x_hi', 's_lo', 's_hi')
+
+
+def empty_rows(n):
+    """Result arrays (T, iA, ix, ia, nsites) of n rows that have not been scanned (gap rows stay so)."""
+    return (np.zeros(n), *(np.full(n, -1, np.int32) for _ in range(3)), np.zeros(n, np.int32))
+
+
+def check_options(world, support, support_drop, refine, refine_steps, null, pvalues):
+    """Refuse option combinations before any work -> (support_drop, refine_steps), checked."""
+    if support is not None:
+        support_drop = support_mod.check_drop(support_drop)
+        if world > 1:
+            raise ValueError('--support runs on one GPU: launch without torchrun (WORLD_SIZE > 1)')
+    if refine is not None:
+        refine_steps = refine_mod.check_steps(refine_steps)
+        if world > 1:
+            raise ValueError('--refine runs on one GPU: launch without torchrun (WORLD_SIZE > 1)')
+    if (null is None) != (pvalues is None):
+        raise ValueError('--null and --pvalues go together')
+    return support_drop, refine_steps
+
+
+def open_outputs(*paths):
+    """Open (truncate) every output file given (None: not asked for).  The reference opens its output before
+    it computes anything (v1:516,551,582,600): a bad path must fail now, not after the scan."""
+    for p in paths:
+        if p is not None:
+            with open(p, 'w'):
+                pass
+
+
+def scan_plan(dev, t, lo, hi, gap, support_drop=None):
+    """The rows of a plan's arrays on one GPU (gap rows left unscanned) and, with ``support_drop``, their
+    support intervals -> (rows, intervals or None)."""
+    rows = empty_rows(len(t))
+    iv = {k: np.full(len(t), -1, np.int32) for k in INTERVAL_KEYS} if support_drop is not None else None
+    live = np.flatnonzero(~gap)
+    if len(live):
+        if support_drop is not None:
+            got, got_iv = scan_with_support(dev, t[live], lo[live], hi[live], support_drop)
+            for k, v in got_iv.items():
+                iv[k][live] = v
+        else:
+            got = dev.run(t[live], lo[live], hi[live])
+        for col, v in zip(rows, got):
+            col[live] = v
+    return rows, iv
+
+
+def write_support(path, plan, order, rows, iv):
+    with open(path, 'w') as fh:
+        fh.write(support_mod.SUPPORT_HEADER)
+        fh.writelines(support_mod.format_support(plan, order, *rows, iv))
+
+
+def write_refine(dev, neutral, sel, K, path, plan, t, lo, hi, rows):
+    """Refine ``rows`` on ``dev`` (refine.py) and write the refine file -> (fine grid, refined rows, moved)."""
+    T, iA, ix, ia, ns = rows
+    grid, refined = refine_mod.refine_rows(dev, neutral, sel, K, t, lo, hi, iA, ix, ia)
+    move = refine_mod.moved(grid, T, iA, ix, ia, refined)
+    with open(path, 'w') as fh:
+        fh.write(HEADER)
+        fh.writelines(refine_mod.format_refined(plan, format_rows(plan, dev.order, *rows), grid, refined, move))
+    print(f'refine (K = {grid.K}): {int(move.sum())} of {int((iA >= 0).sum())} rows with T > 0 moved to a '
+          f'finer grid point')
+    return grid, refined, move
+
+
+def write_pvalues(path, plan, order, rows, gap, null_T):
+    """p-values of ``rows`` against the null CLRs (gap rows NA), written to ``path`` -> p."""
+    p = null_mod.pvalues(np.where(gap, np.nan, rows[0]), null_T)
+    with open(path, 'w') as fh:
+        fh.writelines(null_mod.format_pvalues(plan, order, *rows, p))
+    return p
+
+
 class Scan:
     """Same constructor as the reference class (v1:613); runs the scan and writes ``outfile``.
 
@@ -255,32 +349,11 @@ class Scan:
                  support_drop=support_mod.DEFAULT_DROP, null=None, pvalues=None, refine=None,
                  refine_steps=refine_mod.DEFAULT_STEPS):
         rank, world, local_rank = _world()
-        if support is not None:
-            support_drop = support_mod.check_drop(support_drop)
-            if world > 1:
-                raise ValueError('--support runs on one GPU: launch without torchrun (WORLD_SIZE > 1)')
-        if refine is not None:
-            refine_steps = refine_mod.check_steps(refine_steps)
-            if world > 1:
-                raise ValueError('--refine runs on one GPU: launch without torchrun (WORLD_SIZE > 1)')
-        if (null is None) != (pvalues is None):
-            raise ValueError('--null and --pvalues go together')
+        support_drop, refine_steps = check_options(world, support, support_drop, refine, refine_steps, null, pvalues)
         plan = windows.make_plan(InputData, fixSize=fixSize, r=r, s=s, phys=phys, noCenter=noCenter)
         if rank == 0:
             print('writing output to %s' % (outfile))
-            # the reference opens the output before it computes anything (v1:516,551,582,600): a bad path
-            # must fail now, not after the scan
-            with open(outfile, 'w'):
-                pass
-            if support is not None:
-                with open(support, 'w'):
-                    pass
-            if pvalues is not None:
-                with open(pvalues, 'w'):
-                    pass
-            if refine is not None:
-                with open(refine, 'w'):
-                    pass
+            open_outputs(outfile, support, pvalues, refine)
         setup = None
         if null is not None:
             setup = null_mod.NullSetup(null, InputData, NeutralSFS, NormalizedBetaBinom, Grids, fixSize=fixSize,
@@ -291,30 +364,23 @@ class Scan:
         dev = DeviceScan(InputData, NeutralSFS, NormalizedBetaBinom, Grids, device=device)
         try:
             t, lo, hi, gap = plan.arrays()
-            live = np.flatnonzero(~gap)
-            T = np.zeros(len(plan)); iA = np.full(len(plan), -1, np.int32)
-            ix = iA.copy(); ia = iA.copy(); ns = np.zeros(len(plan), np.int32)
-            iv = {k: np.full(len(plan), -1, np.int32) for k in ('A_lo', 'A_hi', 'x_lo', 'x_hi', 's_lo', 's_hi')}
-            if len(live):
-                if world > 1:
+            if world > 1:
+                live = np.flatnonzero(~gap)
+                rows, iv = empty_rows(len(plan)), None
+                if len(live):
                     got = scan_rows_multi_gpu(dev, t[live], lo[live], hi[live], rank, world, local_rank,
                                               keep_group=setup is not None)
-                elif support is not None:
-                    got, got_iv = scan_with_support(dev, t[live], lo[live], hi[live], support_drop)
-                    for k, v in got_iv.items():
-                        iv[k][live] = v
-                else:
-                    got = dev.run(t[live], lo[live], hi[live])
-                if got is not None:
-                    T[live], iA[live], ix[live], ia[live], ns[live] = got
-            self.results = (T, iA, ix, ia, ns) if rank == 0 else None
+                    if got is not None:
+                        for col, v in zip(rows, got):
+                            col[live] = v
+            else:
+                rows, iv = scan_plan(dev, t, lo, hi, gap, support_drop if support is not None else None)
+            self.results = rows if rank == 0 else None
             if rank == 0:
-                write_scan(outfile, plan, dev.order, T, iA, ix, ia, ns)
+                write_scan(outfile, plan, dev.order, *rows)
                 if support is not None:
                     self.support = iv
-                    with open(support, 'w') as fh:
-                        fh.write(support_mod.SUPPORT_HEADER)
-                        fh.writelines(support_mod.format_support(plan, dev.order, T, iA, ix, ia, ns, iv))
+                    write_support(support, plan, dev.order, rows, iv)
                 if refine is not None:
                     self._refine(dev, NeutralSFS, NormalizedBetaBinom, refine_steps, refine, plan, t, lo, hi)
         finally:
@@ -322,27 +388,17 @@ class Scan:
         if setup is not None:
             null_T = self._scan_null(setup, device, rank, world, local_rank)
             if rank == 0:
-                p = null_mod.pvalues(np.where(gap, np.nan, T), null_T)
-                self.null, self.pvalues = null_T, p
+                self.null = null_T
                 for line in null_mod.summary(null_T, setup.rep, setup.n_replicates):
                     print(line)
-                with open(pvalues, 'w') as fh:
-                    fh.writelines(null_mod.format_pvalues(plan, dev.order, T, iA, ix, ia, ns, p))
+                self.pvalues = write_pvalues(pvalues, plan, dev.order, rows, gap, null_T)
         if rank == 0:
             print(f'{datetime.now()}. Scan finished.')
 
     def _refine(self, dev, neutral, sel, K, path, plan, t, lo, hi):
         """Refine the rows of ``self.results`` on ``dev`` and write the refine file."""
-        T, iA, ix, ia, ns = self.results
-        grid, rows = refine_mod.refine_rows(dev, neutral, sel, K, t, lo, hi, iA, ix, ia)
-        move = refine_mod.moved(grid, T, iA, ix, ia, rows)
-        self.refined, self.refine_grid, self.moved = rows, grid, move
-        with open(path, 'w') as fh:
-            fh.write(HEADER)
-            fh.writelines(refine_mod.format_refined(plan, format_rows(plan, dev.order, T, iA, ix, ia, ns), grid,
-                                                    rows, move))
-        print(f'refine (K = {grid.K}): {int(move.sum())} of {int((iA >= 0).sum())} rows with T > 0 moved to a '
-              f'finer grid point')
+        self.refine_grid, self.refined, self.moved = write_refine(dev, neutral, sel, K, path, plan, t, lo, hi,
+                                                                  self.results)
 
     @staticmethod
     def _scan_null(setup, device, rank, world, local_rank):
@@ -356,3 +412,152 @@ class Scan:
             return ndev.run(setup.t, setup.lo, setup.hi)[0]
         finally:
             ndev.close()
+
+
+def input_list(path):
+    """Inputs of ``--inputList``: the files the list ``path`` names, by the rules of ``null.read_list`` (paths
+    relative to the list's directory, blank and '#' lines skipped).  Every input writes a file named as it is,
+    so two inputs with the same file name are refused.  Raises before any input is read."""
+    paths = null_mod.read_list(path, flag='--inputList', item='input')
+    seen = {}
+    for p in paths:
+        name = os.path.basename(p)
+        if name in seen:
+            raise ValueError(f'--inputList: inputs {seen[name]} and {p} have the same file name {name}; '
+                             f'their outputs would overwrite each other')
+        seen[name] = p
+    return paths
+
+
+def list_outputs(inputs, **dirs):
+    """The files of ``--inputList``: for every directory given (None: option not used), one file per input named
+    as the input -> {option: [paths]}.  Two options naming the same directory, or an output that is one of the
+    inputs, is refused."""
+    files = {k: [os.path.join(d, os.path.basename(p)) for p in inputs] for k, d in dirs.items() if d is not None}
+    out = [os.path.realpath(p) for paths in files.values() for p in paths]
+    if len(set(out)) != len(out):
+        raise ValueError('--inputList: two output options name the same directory')
+    clash = set(out) & {os.path.realpath(p) for p in inputs}
+    if clash:
+        raise ValueError(f'--inputList: output {sorted(clash)[0]} would overwrite an input')
+    return files
+
+
+class GenomeScan:
+    """Scan one input per chromosome (``--inputList``) as one run: one process, one CUDA context, one null.
+
+    ``inputs``: the input paths (``input_list``); ``read(path)`` -> (InputData, NormalizedBetaBinom) of one input,
+    after ``NeutralSFS.get_neut_probs`` of it, as the one-input command line builds them, so that each input keeps
+    the minCount it derives and its own tables.  Every input is loaded as its own problem on its own handle (not
+    one segmented problem: class order and block alignment would differ), and every file it writes is the file a
+    one-input ``Scan`` with the same options writes for it.  ``outdir`` (and ``support``, ``pvalues``, ``refine``
+    when given) are directories; input ``chr7.txt`` writes ``outdir/chr7.txt`` and so on.  Every output file is
+    opened before any input is read.
+
+    One GPU: the inputs are read, scanned and written one after another, with one problem resident at a time.
+    Under torchrun the genome is sharded, not each input: the centres of all inputs are cut into cost-balanced
+    ranges (``scan_seqs_multi_gpu``), each rank loads only the inputs its range touches, one gather brings every
+    row to rank 0, which writes the files.  ``support`` and ``refine`` are one-GPU options, as in ``Scan``.
+
+    ``null``/``pvalues``: the replicates are set up and scanned once (the null depends on the run's flags and
+    spectrum, not on the input: ``null.flags_of``), and every input's p-values come from that pooled null."""
+
+    def __init__(self, inputs, read, NeutralSFS, Grids, outdir, fixSize=False, r=0, s=1, phys=False,
+                 noCenter=False, device=0, support=None, support_drop=support_mod.DEFAULT_DROP, null=None,
+                 pvalues=None, refine=None, refine_steps=refine_mod.DEFAULT_STEPS):
+        rank, world, local_rank = _world()
+        support_drop, refine_steps = check_options(world, support, support_drop, refine, refine_steps, null, pvalues)
+        self.inputs = list(inputs)
+        self.files = list_outputs(self.inputs, out=outdir, support=support, pvalues=pvalues, refine=refine)
+        if rank == 0:
+            print(f'writing {len(self.inputs)} outputs to {outdir}')
+            for paths in self.files.values():
+                open_outputs(*paths)
+        self.kw = dict(fixSize=fixSize, r=r, s=s, phys=phys, noCenter=noCenter)
+        self.read, self.neutral, self.grids, self.null = read, NeutralSFS, Grids, null
+        if world > 1:
+            from .native import device_count
+            self._sharded(local_rank % max(1, device_count()), rank, world, local_rank)
+        else:
+            self._one_gpu(device, support_drop, refine_steps)
+        if rank == 0:
+            print(f'{datetime.now()}. Scan finished.')
+
+    def _null(self, data, sel, device, rank, world, local_rank):
+        """Set up and scan the replicates once -> (NullSetup, null CLRs on rank 0)."""
+        setup = null_mod.NullSetup(self.null, data, self.neutral, sel, self.grids, **self.kw)
+        null_T = Scan._scan_null(setup, device, rank, world, local_rank)
+        if rank == 0:
+            for line in null_mod.summary(null_T, setup.rep, setup.n_replicates):
+                print(line)
+        return setup, null_T
+
+    def _one_gpu(self, device, support_drop, refine_steps):
+        null_T = None
+        for i, path in enumerate(self.inputs):
+            data, sel = self.read(path)
+            if self.null is not None and null_T is None:
+                _, null_T = self._null(data, sel, device, 0, 1, 0)
+            plan = windows.make_plan(data, **self.kw)
+            t, lo, hi, gap = plan.arrays()
+            t0 = time.perf_counter()
+            dev = DeviceScan(data, self.neutral, sel, self.grids, device=device)
+            try:
+                rows, iv = scan_plan(dev, t, lo, hi, gap, support_drop if 'support' in self.files else None)
+                dt = time.perf_counter() - t0
+                write_scan(self.files['out'][i], plan, dev.order, *rows)
+                if iv is not None:
+                    write_support(self.files['support'][i], plan, dev.order, rows, iv)
+                if 'refine' in self.files:
+                    write_refine(dev, self.neutral, sel, refine_steps, self.files['refine'][i], plan, t, lo, hi, rows)
+            finally:
+                dev.close()
+            if null_T is not None:
+                write_pvalues(self.files['pvalues'][i], plan, dev.order, rows, gap, null_T)
+            print(f'{os.path.basename(path)}: {len(plan)} rows, scanned in {dt:.3f} s, written to '
+                  f'{self.files["out"][i]}')
+
+    def _sharded(self, device, rank, world, local_rank):
+        items = []
+        for path in self.inputs:
+            data, sel = self.read(path)
+            plan = windows.make_plan(data, **self.kw)
+            t, lo, hi, gap = plan.arrays()
+            items.append((data, sel, plan, t, lo, hi, gap, np.flatnonzero(~gap)))
+        setup = None
+        if self.null is not None:           # prepared now, scanned after the genome (the process group is kept)
+            setup = null_mod.NullSetup(self.null, items[0][0], self.neutral, items[0][1], self.grids, **self.kw)
+        A = np.array([float(v) for v in GridOrder(self.grids).A])
+        seqs = [(d.genPos, A, t[live], lo[live], hi[live], None) for d, _, _, t, lo, hi, _, live in items]
+
+        def open_dev(i):
+            return DeviceScan(items[i][0], self.neutral, items[i][1], self.grids, device=device)
+
+        t0 = time.perf_counter()
+        got = None
+        if sum(len(s[2]) for s in seqs):
+            got = scan_seqs_multi_gpu(seqs, open_dev, device, rank, world, keep_group=setup is not None,
+                                      release=True)
+        dt = time.perf_counter() - t0
+        null_T = None
+        if setup is not None:
+            null_T = Scan._scan_null(setup, device, rank, world, local_rank)
+        if rank != 0:
+            return
+        if null_T is not None:
+            for line in null_mod.summary(null_T, setup.rep, setup.n_replicates):
+                print(line)
+        print(f'genome: {sum(len(s[2]) for s in seqs)} centres of {len(items)} inputs scanned on {world} ranks '
+              f'in {dt:.3f} s')
+        order = GridOrder(self.grids)
+        o = 0
+        for i, (data, sel, plan, t, lo, hi, gap, live) in enumerate(items):
+            rows = empty_rows(len(plan))
+            if got is not None:
+                for col, v in zip(rows, got):
+                    col[live] = v[o:o + len(live)]
+            o += len(live)
+            write_scan(self.files['out'][i], plan, order, *rows)
+            if null_T is not None:
+                write_pvalues(self.files['pvalues'][i], plan, order, rows, gap, null_T)
+            print(f'{os.path.basename(self.inputs[i])}: {len(plan)} rows, written to {self.files["out"][i]}')

@@ -114,20 +114,66 @@ def gather_rows(rows, counts, rank, world, dist, torch, dst=0):
     return None
 
 
-def scan_sharded(genpos, A, t, lo, hi, rank, world, scan_fn, dist, torch, seg_start=None):
-    """Scan one sequence's centres on `world` ranks and gather the rows on rank 0.
+def genome_costs(seqs):
+    """``centre_costs`` of several sequences, concatenated in sequence order.  ``seqs``: one
+    (genpos, A, t, lo, hi, seg_start) per sequence -> (costs, offs), offs[i] = first centre of sequence i
+    in the concatenated centre list (offs[-1] = all centres)."""
+    costs = [centre_costs(g, t, lo, hi, A, seg) for g, A, t, lo, hi, seg in seqs]
+    offs = np.concatenate(([0], np.cumsum([len(c) for c in costs]))).astype(np.int64)
+    return (np.concatenate(costs) if costs else np.zeros(0)), offs
+
+
+def pieces(offs, b, e):
+    """The sequences a range [b, e) of the concatenated centre list touches -> [(sequence, lb, le)] with
+    [lb, le) a non-empty range of that sequence's own centres, in order.  An empty range touches none."""
+    out = []
+    for i in range(len(offs) - 1):
+        lb, le = max(b, offs[i]), min(e, offs[i + 1])
+        if lb < le:
+            out.append((i, int(lb - offs[i]), int(le - offs[i])))
+    return out
+
+
+def scan_sharded_seqs(seqs, rank, world, scan_fn, dist, torch, device=None):
+    """Scan the centres of several sequences (one per chromosome: a genome) on `world` ranks and gather the
+    rows on rank 0.
+
+    The genome is sharded, not each sequence: the centres of all sequences, laid end to end, are cut into
+    `world` cost-balanced contiguous ranges, so a rank's range may hold the end of one sequence and the
+    start of the next, and a small sequence may lie within one rank's range.  ``seqs`` holds one
+    (genpos, A, t, lo, hi, seg_start) per sequence.  `scan_fn(i, t, lo, hi)` scans a contiguous slice of
+    sequence i's centre list on this rank's device and returns torch tensors (T float64, iA, ix, ia,
+    nsites int32) living on that device; it is called once per sequence the rank's range touches, in order,
+    and never for the others, so a rank needs only those sequences on its device.  A rank whose range is
+    empty sends an empty block made on ``device``.  Returns the five gathered tensors on rank 0 (the
+    concatenated centre list, in order) and None elsewhere.
+    """
+    costs, offs = genome_costs(seqs)
+    parts = partition(costs, world)
+    counts = [e - b for b, e in parts]
+    blocks = []
+    for i, lb, le in pieces(offs, *parts[rank]):
+        t, lo, hi = (np.asarray(a)[lb:le] for a in seqs[i][2:5])
+        blocks.append(pack_rows(*scan_fn(i, t, lo, hi), torch))
+    if not blocks:
+        rows = torch.zeros((0, 6), dtype=torch.int32, device=device)
+    else:
+        rows = blocks[0] if len(blocks) == 1 else torch.cat(blocks, dim=0)
+    got = gather_rows(rows, counts, rank, world, dist, torch)
+    return unpack_rows(got, torch) if got is not None else None
+
+
+def scan_sharded(genpos, A, t, lo, hi, rank, world, scan_fn, dist, torch, seg_start=None, device=None):
+    """Scan one sequence's centres on `world` ranks and gather the rows on rank 0: ``scan_sharded_seqs``
+    with one sequence.
 
     `scan_fn(t, lo, hi)` scans a contiguous slice of the centre list on this rank's device and
     returns torch tensors (T float64, iA, ix, ia, nsites int32) living on that device (the
     product passes ``DeviceScan.run_device``, i.e. ``blmx_scan_device`` on torch's current stream, so the
     rows never leave the GPU before the gather; CPU tests pass the oracle).
     Returns the five gathered tensors on rank 0 (in centre order) and None elsewhere.
-    ``seg_start``: the segment starts of a segmented problem, for the costs.
+    ``seg_start``: the segment starts of a segmented problem, for the costs.  ``device``: where a rank with
+    no centres makes its empty block.
     """
-    costs = centre_costs(genpos, t, lo, hi, A, seg_start)
-    parts = partition(costs, world)
-    counts = [e - b for b, e in parts]
-    b, e = parts[rank]
-    rows = pack_rows(*scan_fn(t[b:e], lo[b:e], hi[b:e]), torch)
-    got = gather_rows(rows, counts, rank, world, dist, torch)
-    return unpack_rows(got, torch) if got is not None else None
+    return scan_sharded_seqs([(genpos, A, t, lo, hi, seg_start)], rank, world,
+                             lambda i, ts, los, his: scan_fn(ts, los, his), dist, torch, device=device)
