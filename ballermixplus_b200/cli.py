@@ -4,8 +4,10 @@ Same flags, defaults, precedence and console messages as the reference's ``main`
 (/root/reference/BalLeRMix+_v1.py:715-802); one extra flag, ``--device``, picks the
 GPU, ``--support`` / ``--supportDrop`` write support intervals of A_hat, x_hat and s_hat (support.py), and
 ``--null`` / ``--pvalues`` write empirical p-values from scans of neutral replicates (null.py), ``--refine``
-/ ``--refineSteps`` write the rows again at the best point of a finer grid around each maximum (refine.py), and
-``--inputList`` scans one input per chromosome in one run (scan.GenomeScan).
+/ ``--refineSteps`` write the rows again at the best point of a finer grid around each maximum (refine.py),
+``--inputList`` scans one input per chromosome in one run (scan.GenomeScan), and ``--regions`` / ``--threshold``
+write one line per run of rows above a CLR cut, with its peak, a support interval for the target's position and,
+with ``--null``, a region p-value (regions.py).
 Differences, all on paths where the reference raises (SURVEY.md appendix A.2,
 DESIGN.md "flags without a reference behaviour"): ``--rangeA``, ``--findPos`` and
 ``--minCount`` with ``--noFreq`` work here.
@@ -21,7 +23,8 @@ from .inputs import InputData
 from .neutral import NeutralSFS
 from .null import read_list
 from .refine import DEFAULT_STEPS, MAX_STEPS, check_steps
-from .scan import GenomeScan, Scan, input_list, list_outputs
+from .regions import check_threshold
+from .scan import REGIONS_NEED_A_CUT, GenomeScan, Scan, check_regions_file, input_list, list_outputs
 from .selection import NormalizedBetaBinom
 from .support import DEFAULT_DROP, check_drop
 
@@ -74,8 +77,8 @@ def build_parser():
                         'composite likelihood: sites are not independent, so they are not calibrated confidence '
                         'intervals. One GPU only (not under torchrun).')
     p.add_argument('--supportDrop', dest='supportDrop', type=_drop, default=DEFAULT_DROP,
-                   help='Drop in T = 2 log LR units that defines the --support intervals. Default '
-                        f'{DEFAULT_DROP} (the chi-square(1) 0.95 quantile).')
+                   help='Drop in T = 2 log LR units that defines the --support intervals and the position '
+                        f'interval of --regions. Default {DEFAULT_DROP} (the chi-square(1) 0.95 quantile).')
     p.add_argument('--null', dest='null', default=None,
                    help='Text file listing neutral replicate inputs, one path per line (relative to the list; '
                         'blank and # lines skipped). Every replicate is scanned with exactly the flags and '
@@ -83,7 +86,7 @@ def build_parser():
                         'pooled replicate CLRs, p = (1 + #{null >= CLR}) / (1 + N_null). The p-values are only as '
                         'good as the neutral model the replicates were simulated under, and they are not '
                         'corrected for multiple testing (the printed quantiles of the per-replicate maximum CLR '
-                        'give a region-level threshold). Needs --pvalues.')
+                        'give a region-level threshold, which --regions applies). Needs --pvalues.')
     p.add_argument('--pvalues', dest='pvalues', default=None,
                    help='With --null: write FILE with physPos, genPos, CLR and p_value per output row.')
     p.add_argument('--refine', dest='refine', default=None,
@@ -102,12 +105,35 @@ def build_parser():
                         'With --getSpect or --getConfig: the helper file of all listed inputs together.')
     p.add_argument('--refineSteps', dest='refineSteps', type=_steps, default=DEFAULT_STEPS,
                    help=f'Fine points per coarse step of --refine, 1 to {MAX_STEPS}. Default {DEFAULT_STEPS}.')
+    p.add_argument('--regions', dest='regions', default=None,
+                   help='Also write FILE: one line per region, a maximal run of consecutive rows (no gap row) with '
+                        'CLR >= the cut, giving its first and last physPos, its row count, its peak row (largest CLR, '
+                        'first on ties) with the peak\'s physPos, genPos, CLR, x_hat, s_hat, A_hat and nSites as the '
+                        'output prints them, and pos_lo / pos_hi: the rows around the peak whose CLR is within '
+                        '--supportDrop of the peak\'s. Each CLR is the maximum over A, x and alpha at its centre, so '
+                        'this is a support interval for the target\'s position, of a composite likelihood: not a '
+                        'calibrated confidence interval. With --null, p_region = (1 + #{replicates whose maximum CLR '
+                        '>= the peak CLR}) / (1 + R): the chance that a neutral replicate holds a row this high, a '
+                        'family-wise p-value only for a sequence of the replicates\' length, not scaled to the '
+                        'genome; NA without --null. The cut is --threshold, or with --null the 0.95 quantile of the '
+                        'per-replicate maximum CLR. With --inputList: one FILE for the whole genome. Works under '
+                        'torchrun; no other output changes.')
+    p.add_argument('--threshold', dest='threshold', type=_threshold, default=None,
+                   help='With --regions: the CLR cut, a finite number > 0. Default with --null: the 0.95 quantile '
+                        'of the per-replicate maximum CLR.')
     return p
 
 
 def _steps(text):
     try:
         return check_steps(text)
+    except ValueError as exc:
+        raise argparse.ArgumentTypeError(str(exc)) from None
+
+
+def _threshold(text):
+    try:
+        return check_threshold(text)
     except ValueError as exc:
         raise argparse.ArgumentTypeError(str(exc)) from None
 
@@ -139,6 +165,10 @@ def main(argv=None):
             read_list(opt.null)             # a bad list fails before any input is read
         except (OSError, ValueError) as exc:
             parser.error(str(exc))
+    if opt.threshold is not None and opt.regions is None:
+        parser.error('--threshold needs --regions')
+    if opt.regions is not None and opt.threshold is None and opt.null is None:
+        parser.error(REGIONS_NEED_A_CUT)
 
     inputs = opt.infile
     if opt.inputList:
@@ -178,7 +208,8 @@ def main(argv=None):
     Scan(data, Neutral, Sel_Probs, grid, opt.outfile, fixSize=opt.size, r=opt.w, s=opt.step,
          phys=opt.phys, noCenter=opt.noCenter, device=opt.device, support=opt.support,
          support_drop=opt.supportDrop, null=opt.null, pvalues=opt.pvalues, refine=opt.refine,
-         refine_steps=opt.refineSteps)
+         refine_steps=opt.refineSteps, regions=opt.regions, threshold=opt.threshold,
+         input_name=os.path.basename(opt.infile))
     print(f'\n{datetime.now()}. Pipeline finished.')
 
 
@@ -198,7 +229,10 @@ def _check_list_mode(parser, opt):
         if d is not None and not os.path.isdir(d):
             parser.error(f'--inputList: {flag} {d} is not an existing directory')
     try:
-        list_outputs(inputs, out=opt.outfile, support=opt.support, pvalues=opt.pvalues, refine=opt.refine)
+        files = list_outputs(inputs, out=opt.outfile, support=opt.support, pvalues=opt.pvalues, refine=opt.refine)
+        if opt.regions is not None:
+            reads = [opt.infile, opt.spectfile] + ([opt.null] + read_list(opt.null) if opt.null else [])
+            check_regions_file(opt.regions, inputs, files, reads)
     except ValueError as exc:
         parser.error(str(exc))
     return inputs
@@ -222,7 +256,8 @@ def _main_list(opt, inputs):
     print('\n%s. Start computing likelihood raito...' % (datetime.now()))
     GenomeScan(inputs, read, Neutral, grid, opt.outfile, fixSize=opt.size, r=opt.w, s=opt.step, phys=opt.phys,
                noCenter=opt.noCenter, device=opt.device, support=opt.support, support_drop=opt.supportDrop,
-               null=opt.null, pvalues=opt.pvalues, refine=opt.refine, refine_steps=opt.refineSteps)
+               null=opt.null, pvalues=opt.pvalues, refine=opt.refine, refine_steps=opt.refineSteps,
+               regions=opt.regions, threshold=opt.threshold)
     print(f'\n{datetime.now()}. Pipeline finished.')
 
 

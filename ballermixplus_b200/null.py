@@ -196,14 +196,22 @@ def format_pvalues(plan, order, T, iA, ix, ia, ns, p):
     return lines
 
 
-def summary(null, rep, n_replicates):
-    """Console lines: replicate and row counts, and the QUANTILES of the null CLR and of the per-replicate
-    maximum CLR."""
+def replicate_maxima(null, rep, n_replicates):
+    """The maximum CLR of every replicate that has one: ``null`` the null CLRs, ``rep`` their replicates.  NaN
+    values are left out; a replicate without a row (or with NaN rows only) has no maximum and is dropped."""
     null = np.asarray(null, dtype=np.float64)
     ok = ~np.isnan(null)
     mx = np.full(n_replicates, -np.inf)
     np.maximum.at(mx, np.asarray(rep)[ok], null[ok])
-    mx = mx[mx > -np.inf]                         # replicates without a row have no maximum
+    return mx[mx > -np.inf]
+
+
+def summary(null, rep, n_replicates):
+    """Console lines: replicate and row counts, and the QUANTILES of the null CLR and of the per-replicate
+    maximum CLR (``replicate_maxima``)."""
+    null = np.asarray(null, dtype=np.float64)
+    ok = ~np.isnan(null)
+    mx = replicate_maxima(null, rep, n_replicates)
 
     def q(v):
         return ', '.join(f'{k}: {np.quantile(v, k):.6g}' for k in QUANTILES) if len(v) else 'none'

@@ -13,7 +13,7 @@ from datetime import datetime
 
 import numpy as np
 
-from . import fastio, null as null_mod, refine as refine_mod, support as support_mod, windows
+from . import fastio, null as null_mod, refine as refine_mod, regions as regions_mod, support as support_mod, windows
 from .native import Scanner
 from .problem import GridOrder, build_problem
 
@@ -257,19 +257,29 @@ def empty_rows(n):
     return (np.zeros(n), *(np.full(n, -1, np.int32) for _ in range(3)), np.zeros(n, np.int32))
 
 
-def check_options(world, support, support_drop, refine, refine_steps, null, pvalues):
-    """Refuse option combinations before any work -> (support_drop, refine_steps), checked."""
-    if support is not None:
+def check_options(world, support, support_drop, refine, refine_steps, null, pvalues, regions=None, threshold=None):
+    """Refuse option combinations before any work -> (support_drop, refine_steps, threshold), checked."""
+    if support is not None or regions is not None:
         support_drop = support_mod.check_drop(support_drop)
-        if world > 1:
-            raise ValueError('--support runs on one GPU: launch without torchrun (WORLD_SIZE > 1)')
+    if support is not None and world > 1:
+        raise ValueError('--support runs on one GPU: launch without torchrun (WORLD_SIZE > 1)')
     if refine is not None:
         refine_steps = refine_mod.check_steps(refine_steps)
         if world > 1:
             raise ValueError('--refine runs on one GPU: launch without torchrun (WORLD_SIZE > 1)')
     if (null is None) != (pvalues is None):
         raise ValueError('--null and --pvalues go together')
-    return support_drop, refine_steps
+    if threshold is not None:
+        if regions is None:
+            raise ValueError('--threshold needs --regions')
+        threshold = regions_mod.check_threshold(threshold)
+    if regions is not None and threshold is None and null is None:
+        raise ValueError(REGIONS_NEED_A_CUT)
+    return support_drop, refine_steps, threshold
+
+
+REGIONS_NEED_A_CUT = ('--regions needs a cut: --threshold C, or --null (the 0.95 quantile of the per-replicate '
+                      'maximum CLR)')
 
 
 def open_outputs(*paths):
@@ -342,18 +352,25 @@ class Scan:
 
     ``refine`` (a path): also write ``outfile`` again with every row with T > 0 replaced by the best point of a
     grid ``refine_steps`` times finer inside a box around its maximum, where that point beats the row's CLR
-    (refine.py).  One GPU only.  ``outfile``, the support and the p-value files stay on the coarse grid."""
+    (refine.py).  One GPU only.  ``outfile``, the support and the p-value files stay on the coarse grid.
+
+    ``regions`` (a path): also write one line per run of rows with CLR >= the cut, with its peak, the position
+    support interval at drop ``support_drop`` and, with ``null``, a region p-value (regions.py).  The cut is
+    ``threshold``, or without it the 0.95 quantile of the per-replicate maximum CLR of ``null``.  ``input_name``
+    fills the file's first column (default: the file name of ``outfile``).  Works under torchrun; no other file
+    changes."""
 
     def __init__(self, InputData, NeutralSFS, NormalizedBetaBinom, Grids, outfile, fixSize=False,
                  r=0, s=1, phys=False, noCenter=False, device=0, support=None,
                  support_drop=support_mod.DEFAULT_DROP, null=None, pvalues=None, refine=None,
-                 refine_steps=refine_mod.DEFAULT_STEPS):
+                 refine_steps=refine_mod.DEFAULT_STEPS, regions=None, threshold=None, input_name=None):
         rank, world, local_rank = _world()
-        support_drop, refine_steps = check_options(world, support, support_drop, refine, refine_steps, null, pvalues)
+        support_drop, refine_steps, threshold = check_options(world, support, support_drop, refine, refine_steps,
+                                                              null, pvalues, regions, threshold)
         plan = windows.make_plan(InputData, fixSize=fixSize, r=r, s=s, phys=phys, noCenter=noCenter)
         if rank == 0:
             print('writing output to %s' % (outfile))
-            open_outputs(outfile, support, pvalues, refine)
+            open_outputs(outfile, support, pvalues, refine, regions)
         setup = None
         if null is not None:
             setup = null_mod.NullSetup(null, InputData, NeutralSFS, NormalizedBetaBinom, Grids, fixSize=fixSize,
@@ -385,6 +402,7 @@ class Scan:
                     self._refine(dev, NeutralSFS, NormalizedBetaBinom, refine_steps, refine, plan, t, lo, hi)
         finally:
             dev.close()
+        maxima = None
         if setup is not None:
             null_T = self._scan_null(setup, device, rank, world, local_rank)
             if rank == 0:
@@ -392,6 +410,12 @@ class Scan:
                 for line in null_mod.summary(null_T, setup.rep, setup.n_replicates):
                     print(line)
                 self.pvalues = write_pvalues(pvalues, plan, dev.order, rows, gap, null_T)
+                maxima = null_mod.replicate_maxima(null_T, setup.rep, setup.n_replicates)
+        if regions is not None and rank == 0:
+            cut, source = regions_mod.cut_of(threshold, maxima)
+            name = os.path.basename(outfile) if input_name is None else input_name
+            self.regions = regions_mod.region_lines(name, plan, dev.order, rows, gap, cut, support_drop, maxima)
+            print(regions_mod.write_regions(regions, [self.regions], cut, source, support_drop))
         if rank == 0:
             print(f'{datetime.now()}. Scan finished.')
 
@@ -443,6 +467,20 @@ def list_outputs(inputs, **dirs):
     return files
 
 
+def check_regions_file(path, inputs, files, reads=()):
+    """``--regions`` of ``--inputList`` names one file for the whole genome: refused when it is a directory, when
+    its directory does not exist, or when it is a file the run reads (an input, ``reads``) or writes (``files``,
+    from ``list_outputs``)."""
+    if os.path.isdir(path):
+        raise ValueError(f'--inputList: --regions {path} is a directory; it names one file for the whole genome')
+    parent = os.path.dirname(os.path.abspath(path))
+    if not os.path.isdir(parent):
+        raise ValueError(f'--inputList: --regions {path}: directory {parent} does not exist')
+    taken = {os.path.realpath(p) for p in list(inputs) + list(reads) + [f for fs in files.values() for f in fs]}
+    if os.path.realpath(path) in taken:
+        raise ValueError(f'--inputList: --regions {path} is a file this run reads or writes')
+
+
 class GenomeScan:
     """Scan one input per chromosome (``--inputList``) as one run: one process, one CUDA context, one null.
 
@@ -460,27 +498,38 @@ class GenomeScan:
     row to rank 0, which writes the files.  ``support`` and ``refine`` are one-GPU options, as in ``Scan``.
 
     ``null``/``pvalues``: the replicates are set up and scanned once (the null depends on the run's flags and
-    spectrum, not on the input: ``null.flags_of``), and every input's p-values come from that pooled null."""
+    spectrum, not on the input: ``null.flags_of``), and every input's p-values come from that pooled null.
+
+    ``regions`` (a path, not a directory) and ``threshold``: one regions file for the whole genome (``Scan``), the
+    lines of every input in input order, collected as its rows become available and written at the end."""
 
     def __init__(self, inputs, read, NeutralSFS, Grids, outdir, fixSize=False, r=0, s=1, phys=False,
                  noCenter=False, device=0, support=None, support_drop=support_mod.DEFAULT_DROP, null=None,
-                 pvalues=None, refine=None, refine_steps=refine_mod.DEFAULT_STEPS):
+                 pvalues=None, refine=None, refine_steps=refine_mod.DEFAULT_STEPS, regions=None, threshold=None):
         rank, world, local_rank = _world()
-        support_drop, refine_steps = check_options(world, support, support_drop, refine, refine_steps, null, pvalues)
+        support_drop, refine_steps, threshold = check_options(world, support, support_drop, refine, refine_steps,
+                                                              null, pvalues, regions, threshold)
         self.inputs = list(inputs)
         self.files = list_outputs(self.inputs, out=outdir, support=support, pvalues=pvalues, refine=refine)
+        if regions is not None:
+            check_regions_file(regions, self.inputs, self.files)
         if rank == 0:
             print(f'writing {len(self.inputs)} outputs to {outdir}')
             for paths in self.files.values():
                 open_outputs(*paths)
+            open_outputs(regions)
         self.kw = dict(fixSize=fixSize, r=r, s=s, phys=phys, noCenter=noCenter)
         self.read, self.neutral, self.grids, self.null = read, NeutralSFS, Grids, null
+        self.region_file, self.threshold, self.drop = regions, threshold, support_drop
+        self.maxima, self.cut, self.regions = None, None, []
         if world > 1:
             from .native import device_count
             self._sharded(local_rank % max(1, device_count()), rank, world, local_rank)
         else:
             self._one_gpu(device, support_drop, refine_steps)
         if rank == 0:
+            if regions is not None:
+                print(regions_mod.write_regions(regions, self.regions, *self.cut, support_drop))
             print(f'{datetime.now()}. Scan finished.')
 
     def _null(self, data, sel, device, rank, world, local_rank):
@@ -488,9 +537,23 @@ class GenomeScan:
         setup = null_mod.NullSetup(self.null, data, self.neutral, sel, self.grids, **self.kw)
         null_T = Scan._scan_null(setup, device, rank, world, local_rank)
         if rank == 0:
-            for line in null_mod.summary(null_T, setup.rep, setup.n_replicates):
-                print(line)
+            self._null_summary(setup, null_T)
         return setup, null_T
+
+    def _null_summary(self, setup, null_T):
+        """Print the null's quantiles and keep its per-replicate maxima (the regions' cut and p-values)."""
+        for line in null_mod.summary(null_T, setup.rep, setup.n_replicates):
+            print(line)
+        self.maxima = null_mod.replicate_maxima(null_T, setup.rep, setup.n_replicates)
+
+    def _add_regions(self, path, plan, order, rows, gap):
+        """Collect the regions of one input (``--regions``); the null, if any, has been scanned."""
+        if self.region_file is None:
+            return
+        if self.cut is None:
+            self.cut = regions_mod.cut_of(self.threshold, self.maxima)
+        self.regions.append(regions_mod.region_lines(os.path.basename(path), plan, order, rows, gap, self.cut[0],
+                                                     self.drop, self.maxima))
 
     def _one_gpu(self, device, support_drop, refine_steps):
         null_T = None
@@ -514,6 +577,7 @@ class GenomeScan:
                 dev.close()
             if null_T is not None:
                 write_pvalues(self.files['pvalues'][i], plan, dev.order, rows, gap, null_T)
+            self._add_regions(path, plan, dev.order, rows, gap)
             print(f'{os.path.basename(path)}: {len(plan)} rows, scanned in {dt:.3f} s, written to '
                   f'{self.files["out"][i]}')
 
@@ -545,8 +609,7 @@ class GenomeScan:
         if rank != 0:
             return
         if null_T is not None:
-            for line in null_mod.summary(null_T, setup.rep, setup.n_replicates):
-                print(line)
+            self._null_summary(setup, null_T)
         print(f'genome: {sum(len(s[2]) for s in seqs)} centres of {len(items)} inputs scanned on {world} ranks '
               f'in {dt:.3f} s')
         order = GridOrder(self.grids)
@@ -560,4 +623,5 @@ class GenomeScan:
             write_scan(self.files['out'][i], plan, order, *rows)
             if null_T is not None:
                 write_pvalues(self.files['pvalues'][i], plan, order, rows, gap, null_T)
+            self._add_regions(self.inputs[i], plan, order, rows, gap)
             print(f'{os.path.basename(self.inputs[i])}: {len(plan)} rows, written to {self.files["out"][i]}')

@@ -50,6 +50,12 @@ class ScanPlan:
             return [f'{v}' for v in self.site_gen]
         return self._f1
 
+    def text(self, j):
+        """(physPos, genPos) text of non-gap row j, as ``f0[j]``, ``f1[j]`` give it, without formatting every row."""
+        if self.site_phys is not None:
+            return f'{self.site_phys[j]}', f'{self.site_gen[j]}'
+        return self._f0[j], self._f1[j]
+
     def add_gap(self, line):
         self.t.append(0.); self.lo.append(0); self.hi.append(-1)
         self._f0.append(line); self._f1.append(''); self.gap.append(True)
