@@ -7,7 +7,8 @@ GPU, ``--support`` / ``--supportDrop`` write support intervals of A_hat, x_hat a
 / ``--refineSteps`` write the rows again at the best point of a finer grid around each maximum (refine.py),
 ``--inputList`` scans one input per chromosome in one run (scan.GenomeScan), and ``--regions`` / ``--threshold``
 write one line per run of rows above a CLR cut, with its peak, a support interval for the target's position and,
-with ``--null``, a region p-value (regions.py).
+with ``--null``, a region p-value (regions.py), and ``--targets`` scans only the rows whose centre lies in listed
+intervals, every output a line-for-line subset of the full scan's (targets.py).
 Differences, all on paths where the reference raises (SURVEY.md appendix A.2,
 DESIGN.md "flags without a reference behaviour"): ``--rangeA``, ``--findPos`` and
 ``--minCount`` with ``--noFreq`` work here.
@@ -24,9 +25,10 @@ from .neutral import NeutralSFS
 from .null import read_list
 from .refine import DEFAULT_STEPS, MAX_STEPS, check_steps
 from .regions import check_threshold
-from .scan import REGIONS_NEED_A_CUT, GenomeScan, Scan, check_regions_file, input_list, list_outputs
+from .scan import REGIONS_NEED_A_CUT, GenomeScan, Scan, check_regions_file, input_list, list_outputs, names_one_of
 from .selection import NormalizedBetaBinom
 from .support import DEFAULT_DROP, check_drop
+from .targets import read_targets
 
 
 def build_parser():
@@ -117,10 +119,21 @@ def build_parser():
                         'family-wise p-value only for a sequence of the replicates\' length, not scaled to the '
                         'genome; NA without --null. The cut is --threshold, or with --null the 0.95 quantile of the '
                         'per-replicate maximum CLR. With --inputList: one FILE for the whole genome. Works under '
-                        'torchrun; no other output changes.')
+                        'torchrun; no other output changes. With --targets, a row that is not kept ends a region and '
+                        'stops a position interval, as a gap row does, so regions are cut at the target edges.')
     p.add_argument('--threshold', dest='threshold', type=_threshold, default=None,
                    help='With --regions: the CLR cut, a finite number > 0. Default with --null: the 0.95 quantile '
                         'of the per-replicate maximum CLR.')
+    p.add_argument('--targets', dest='targets', default=None,
+                   help='Scan only the rows whose physPos lies in a target of FILE: one target per line, "name start '
+                        'end", name the input\'s file name (with --inputList, of a listed input), start and end '
+                        'inclusive physPos values compared as numbers; blank and # lines, a header line starting with '
+                        '"input" and fields after the third are skipped, so a --regions file is a targets file as '
+                        'written. Targets may overlap. Every output file holds the header and, in order, exactly the '
+                        'lines the same run without --targets writes at the kept rows (DESIGN.md §3.13). --regions '
+                        'is the exception: a row that is not kept ends a region and stops a '
+                        'position interval, as a gap row does, so a region or interval that reaches the first or last '
+                        'kept row of a target is cut there. The --null replicates are still scanned in full.')
     return p
 
 
@@ -173,6 +186,7 @@ def main(argv=None):
     inputs = opt.infile
     if opt.inputList:
         inputs = _check_list_mode(parser, opt)
+    targets = _check_targets(parser, opt, inputs)
 
     if opt.getSpec:
         print('You\'ve chosen to generate site frequency spectrum...')
@@ -185,7 +199,7 @@ def main(argv=None):
         getConfig(inputs, opt.spectfile)
         sys.exit()
     if opt.inputList:
-        _main_list(opt, inputs)
+        _main_list(opt, inputs, targets)
         return
 
     print(f'\n{datetime.now()}. Reading input from {opt.infile}')
@@ -209,7 +223,7 @@ def main(argv=None):
          phys=opt.phys, noCenter=opt.noCenter, device=opt.device, support=opt.support,
          support_drop=opt.supportDrop, null=opt.null, pvalues=opt.pvalues, refine=opt.refine,
          refine_steps=opt.refineSteps, regions=opt.regions, threshold=opt.threshold,
-         input_name=os.path.basename(opt.infile))
+         input_name=os.path.basename(opt.infile), targets=targets)
     print(f'\n{datetime.now()}. Pipeline finished.')
 
 
@@ -238,7 +252,29 @@ def _check_list_mode(parser, opt):
     return inputs
 
 
-def _main_list(opt, inputs):
+def _check_targets(parser, opt, inputs):
+    """``--targets``: the parsed targets file (None without the option).  Refused before any input is read with
+    --getSpect or --getConfig, when the run writes the file, and when the file is bad (targets.read_targets)."""
+    if opt.targets is None:
+        return None
+    if opt.getSpec or opt.getConfig:
+        parser.error('--targets selects the rows of a scan; --getSpect and --getConfig do not scan')
+    if opt.inputList:
+        names = [os.path.basename(p) for p in inputs]
+        files = list_outputs(inputs, out=opt.outfile, support=opt.support, pvalues=opt.pvalues, refine=opt.refine)
+        written = [f for fs in files.values() for f in fs] + [opt.regions]
+    else:
+        names = [os.path.basename(opt.infile)]
+        written = [opt.outfile, opt.support, opt.pvalues, opt.refine, opt.regions]
+    if names_one_of(opt.targets, written):
+        parser.error(f'--targets {opt.targets} is a file this run writes')
+    try:
+        return read_targets(opt.targets, names)
+    except ValueError as exc:
+        parser.error(str(exc))
+
+
+def _main_list(opt, inputs, targets=None):
     """One run over every listed input (scan.GenomeScan), each read and tabulated as the one-input run reads it."""
     print(f'\n{datetime.now()}. {len(inputs)} inputs listed in {opt.infile}')
     Neutral = NeutralSFS(opt.spectfile, opt.nofreq, opt.MAF, opt.nosub)
@@ -257,7 +293,7 @@ def _main_list(opt, inputs):
     GenomeScan(inputs, read, Neutral, grid, opt.outfile, fixSize=opt.size, r=opt.w, s=opt.step, phys=opt.phys,
                noCenter=opt.noCenter, device=opt.device, support=opt.support, support_drop=opt.supportDrop,
                null=opt.null, pvalues=opt.pvalues, refine=opt.refine, refine_steps=opt.refineSteps,
-               regions=opt.regions, threshold=opt.threshold)
+               regions=opt.regions, threshold=opt.threshold, targets=targets)
     print(f'\n{datetime.now()}. Pipeline finished.')
 
 

@@ -14,6 +14,7 @@ from datetime import datetime
 import numpy as np
 
 from . import fastio, null as null_mod, refine as refine_mod, regions as regions_mod, support as support_mod, windows
+from . import targets as targets_mod
 from .native import Scanner
 from .problem import GridOrder, build_problem
 
@@ -81,6 +82,17 @@ class DeviceScan:
 
     def close(self):
         self.scanner.close()
+
+
+class Unloaded:
+    """Stands in for the DeviceScan of an input none of whose rows is scanned (``--targets`` keeps no row of it that
+    is not a gap row): the writers need only its grid order, so nothing is loaded on a GPU."""
+
+    def __init__(self, grids):
+        self.order = GridOrder(grids)
+
+    def close(self):
+        pass
 
 
 _cache = {}       # 'objs': the four host objects of the resident problem (strong references), 'dev': its DeviceScan
@@ -292,8 +304,8 @@ def open_outputs(*paths):
 
 
 def scan_plan(dev, t, lo, hi, gap, support_drop=None):
-    """The rows of a plan's arrays on one GPU (gap rows left unscanned) and, with ``support_drop``, their
-    support intervals -> (rows, intervals or None)."""
+    """The rows of a plan's arrays on one GPU (gap rows, and rows ``--targets`` skips, passed in ``gap``, left
+    unscanned) and, with ``support_drop``, their support intervals -> (rows, intervals or None)."""
     rows = empty_rows(len(t))
     iv = {k: np.full(len(t), -1, np.int32) for k in INTERVAL_KEYS} if support_drop is not None else None
     live = np.flatnonzero(~gap)
@@ -307,6 +319,22 @@ def scan_plan(dev, t, lo, hi, gap, support_drop=None):
         for col, v in zip(rows, got):
             col[live] = v
     return rows, iv
+
+
+def select_rows(keep, plan, arrays, rows, iv):
+    """What a run writes -> (plan, arrays, rows, intervals): everything when ``keep`` is None, else only the rows
+    ``keep`` selects (``--targets``), in order.  ``arrays`` = (t, lo, hi, gap) of ``plan``, ``iv`` the support
+    intervals or None."""
+    if keep is None:
+        return plan, arrays, rows, iv
+    idx = np.flatnonzero(keep)
+    return (plan.take(idx), tuple(a[idx] for a in arrays), tuple(c[idx] for c in rows),
+            None if iv is None else {k: v[idx] for k, v in iv.items()})
+
+
+def skipped(gap, keep):
+    """Rows not scanned: the gap rows, and with ``--targets`` (``keep``) every row it does not keep."""
+    return gap if keep is None else gap | ~keep
 
 
 def write_support(path, plan, order, rows, iv):
@@ -358,19 +386,29 @@ class Scan:
     support interval at drop ``support_drop`` and, with ``null``, a region p-value (regions.py).  The cut is
     ``threshold``, or without it the 0.95 quantile of the per-replicate maximum CLR of ``null``.  ``input_name``
     fills the file's first column (default: the file name of ``outfile``).  Works under torchrun; no other file
-    changes."""
+    changes.
+
+    ``targets`` (a ``targets.Targets``): scan only the rows whose physPos lies in a target of the input named
+    ``input_name``; every file then holds the header and, in order, exactly the lines of the full run at those rows
+    (``results`` too holds those rows only).  A row not kept ends a region and stops a position interval, as a gap
+    row does."""
 
     def __init__(self, InputData, NeutralSFS, NormalizedBetaBinom, Grids, outfile, fixSize=False,
                  r=0, s=1, phys=False, noCenter=False, device=0, support=None,
                  support_drop=support_mod.DEFAULT_DROP, null=None, pvalues=None, refine=None,
-                 refine_steps=refine_mod.DEFAULT_STEPS, regions=None, threshold=None, input_name=None):
+                 refine_steps=refine_mod.DEFAULT_STEPS, regions=None, threshold=None, input_name=None,
+                 targets=None):
         rank, world, local_rank = _world()
         support_drop, refine_steps, threshold = check_options(world, support, support_drop, refine, refine_steps,
                                                               null, pvalues, regions, threshold)
         plan = windows.make_plan(InputData, fixSize=fixSize, r=r, s=s, phys=phys, noCenter=noCenter)
+        name = os.path.basename(outfile) if input_name is None else input_name
+        keep = None if targets is None else targets.keep(name, plan)
         if rank == 0:
             print('writing output to %s' % (outfile))
             open_outputs(outfile, support, pvalues, refine, regions)
+            if keep is not None:
+                print(targets_mod.kept_line(name, keep))
         setup = None
         if null is not None:
             setup = null_mod.NullSetup(null, InputData, NeutralSFS, NormalizedBetaBinom, Grids, fixSize=fixSize,
@@ -378,11 +416,15 @@ class Scan:
         if world > 1:
             from .native import device_count
             device = local_rank % max(1, device_count())
-        dev = DeviceScan(InputData, NeutralSFS, NormalizedBetaBinom, Grids, device=device)
+        t, lo, hi, gap = plan.arrays()
+        skip = skipped(gap, keep)
+        if keep is not None and skip.all():
+            dev = Unloaded(Grids)
+        else:
+            dev = DeviceScan(InputData, NeutralSFS, NormalizedBetaBinom, Grids, device=device)
         try:
-            t, lo, hi, gap = plan.arrays()
             if world > 1:
-                live = np.flatnonzero(~gap)
+                live = np.flatnonzero(~skip)
                 rows, iv = empty_rows(len(plan)), None
                 if len(live):
                     got = scan_rows_multi_gpu(dev, t[live], lo[live], hi[live], rank, world, local_rank,
@@ -391,15 +433,16 @@ class Scan:
                         for col, v in zip(rows, got):
                             col[live] = v
             else:
-                rows, iv = scan_plan(dev, t, lo, hi, gap, support_drop if support is not None else None)
-            self.results = rows if rank == 0 else None
+                rows, iv = scan_plan(dev, t, lo, hi, skip, support_drop if support is not None else None)
+            wplan, (wt, wlo, whi, wgap), wrows, wiv = select_rows(keep, plan, (t, lo, hi, gap), rows, iv)
+            self.results = wrows if rank == 0 else None
             if rank == 0:
-                write_scan(outfile, plan, dev.order, *rows)
+                write_scan(outfile, wplan, dev.order, *wrows)
                 if support is not None:
-                    self.support = iv
-                    write_support(support, plan, dev.order, rows, iv)
+                    self.support = wiv
+                    write_support(support, wplan, dev.order, wrows, wiv)
                 if refine is not None:
-                    self._refine(dev, NeutralSFS, NormalizedBetaBinom, refine_steps, refine, plan, t, lo, hi)
+                    self._refine(dev, NeutralSFS, NormalizedBetaBinom, refine_steps, refine, wplan, wt, wlo, whi)
         finally:
             dev.close()
         maxima = None
@@ -409,12 +452,11 @@ class Scan:
                 self.null = null_T
                 for line in null_mod.summary(null_T, setup.rep, setup.n_replicates):
                     print(line)
-                self.pvalues = write_pvalues(pvalues, plan, dev.order, rows, gap, null_T)
+                self.pvalues = write_pvalues(pvalues, wplan, dev.order, wrows, wgap, null_T)
                 maxima = null_mod.replicate_maxima(null_T, setup.rep, setup.n_replicates)
         if regions is not None and rank == 0:
             cut, source = regions_mod.cut_of(threshold, maxima)
-            name = os.path.basename(outfile) if input_name is None else input_name
-            self.regions = regions_mod.region_lines(name, plan, dev.order, rows, gap, cut, support_drop, maxima)
+            self.regions = regions_mod.region_lines(name, plan, dev.order, rows, skip, cut, support_drop, maxima)
             print(regions_mod.write_regions(regions, [self.regions], cut, source, support_drop))
         if rank == 0:
             print(f'{datetime.now()}. Scan finished.')
@@ -476,9 +518,14 @@ def check_regions_file(path, inputs, files, reads=()):
     parent = os.path.dirname(os.path.abspath(path))
     if not os.path.isdir(parent):
         raise ValueError(f'--inputList: --regions {path}: directory {parent} does not exist')
-    taken = {os.path.realpath(p) for p in list(inputs) + list(reads) + [f for fs in files.values() for f in fs]}
-    if os.path.realpath(path) in taken:
+    if names_one_of(path, list(inputs) + list(reads) + [f for fs in files.values() for f in fs]):
         raise ValueError(f'--inputList: --regions {path} is a file this run reads or writes')
+
+
+def names_one_of(path, paths):
+    """True when ``path`` names the same file as one of ``paths`` (None entries ignored), links and relative parts
+    resolved."""
+    return os.path.realpath(path) in {os.path.realpath(p) for p in paths if p is not None}
 
 
 class GenomeScan:
@@ -501,11 +548,16 @@ class GenomeScan:
     spectrum, not on the input: ``null.flags_of``), and every input's p-values come from that pooled null.
 
     ``regions`` (a path, not a directory) and ``threshold``: one regions file for the whole genome (``Scan``), the
-    lines of every input in input order, collected as its rows become available and written at the end."""
+    lines of every input in input order, collected as its rows become available and written at the end.
+
+    ``targets`` (a ``targets.Targets``, inputs named by file name): each input keeps only the rows in its targets, as
+    in ``Scan``; the centres of the kept rows alone are scanned (and sharded under torchrun), and an input with no
+    kept row to scan is read and planned but never loaded on a GPU."""
 
     def __init__(self, inputs, read, NeutralSFS, Grids, outdir, fixSize=False, r=0, s=1, phys=False,
                  noCenter=False, device=0, support=None, support_drop=support_mod.DEFAULT_DROP, null=None,
-                 pvalues=None, refine=None, refine_steps=refine_mod.DEFAULT_STEPS, regions=None, threshold=None):
+                 pvalues=None, refine=None, refine_steps=refine_mod.DEFAULT_STEPS, regions=None, threshold=None,
+                 targets=None):
         rank, world, local_rank = _world()
         support_drop, refine_steps, threshold = check_options(world, support, support_drop, refine, refine_steps,
                                                               null, pvalues, regions, threshold)
@@ -522,6 +574,7 @@ class GenomeScan:
         self.read, self.neutral, self.grids, self.null = read, NeutralSFS, Grids, null
         self.region_file, self.threshold, self.drop = regions, threshold, support_drop
         self.maxima, self.cut, self.regions = None, None, []
+        self.targets, self.kept = targets, []
         if world > 1:
             from .native import device_count
             self._sharded(local_rank % max(1, device_count()), rank, world, local_rank)
@@ -530,6 +583,9 @@ class GenomeScan:
         if rank == 0:
             if regions is not None:
                 print(regions_mod.write_regions(regions, self.regions, *self.cut, support_drop))
+            if targets is not None:
+                print(f'--targets: {sum(k for k, _ in self.kept)} of {sum(n for _, n in self.kept)} planned rows '
+                      f'kept in {sum(1 for k, _ in self.kept if k)} of {len(self.kept)} inputs')
             print(f'{datetime.now()}. Scan finished.')
 
     def _null(self, data, sel, device, rank, world, local_rank):
@@ -555,29 +611,44 @@ class GenomeScan:
         self.regions.append(regions_mod.region_lines(os.path.basename(path), plan, order, rows, gap, self.cut[0],
                                                      self.drop, self.maxima))
 
+    def _plan(self, path, data):
+        """-> (plan, t, lo, hi, gap, keep, skip) of one input (``keep`` None without ``--targets``)."""
+        plan = windows.make_plan(data, **self.kw)
+        t, lo, hi, gap = plan.arrays()
+        keep = None
+        if self.targets is not None:
+            keep = self.targets.keep(os.path.basename(path), plan)
+            self.kept.append((int(np.count_nonzero(keep)), len(plan)))
+            print(targets_mod.kept_line(os.path.basename(path), keep))
+        return plan, t, lo, hi, gap, keep, skipped(gap, keep)
+
     def _one_gpu(self, device, support_drop, refine_steps):
         null_T = None
         for i, path in enumerate(self.inputs):
             data, sel = self.read(path)
             if self.null is not None and null_T is None:
                 _, null_T = self._null(data, sel, device, 0, 1, 0)
-            plan = windows.make_plan(data, **self.kw)
-            t, lo, hi, gap = plan.arrays()
+            plan, t, lo, hi, gap, keep, skip = self._plan(path, data)
             t0 = time.perf_counter()
-            dev = DeviceScan(data, self.neutral, sel, self.grids, device=device)
+            if keep is not None and skip.all():
+                dev = Unloaded(self.grids)
+            else:
+                dev = DeviceScan(data, self.neutral, sel, self.grids, device=device)
             try:
-                rows, iv = scan_plan(dev, t, lo, hi, gap, support_drop if 'support' in self.files else None)
+                rows, iv = scan_plan(dev, t, lo, hi, skip, support_drop if 'support' in self.files else None)
                 dt = time.perf_counter() - t0
-                write_scan(self.files['out'][i], plan, dev.order, *rows)
-                if iv is not None:
-                    write_support(self.files['support'][i], plan, dev.order, rows, iv)
+                wplan, (wt, wlo, whi, wgap), wrows, wiv = select_rows(keep, plan, (t, lo, hi, gap), rows, iv)
+                write_scan(self.files['out'][i], wplan, dev.order, *wrows)
+                if wiv is not None:
+                    write_support(self.files['support'][i], wplan, dev.order, wrows, wiv)
                 if 'refine' in self.files:
-                    write_refine(dev, self.neutral, sel, refine_steps, self.files['refine'][i], plan, t, lo, hi, rows)
+                    write_refine(dev, self.neutral, sel, refine_steps, self.files['refine'][i], wplan, wt, wlo, whi,
+                                 wrows)
             finally:
                 dev.close()
             if null_T is not None:
-                write_pvalues(self.files['pvalues'][i], plan, dev.order, rows, gap, null_T)
-            self._add_regions(path, plan, dev.order, rows, gap)
+                write_pvalues(self.files['pvalues'][i], wplan, dev.order, wrows, wgap, null_T)
+            self._add_regions(path, plan, dev.order, rows, skip)
             print(f'{os.path.basename(path)}: {len(plan)} rows, scanned in {dt:.3f} s, written to '
                   f'{self.files["out"][i]}')
 
@@ -585,14 +656,14 @@ class GenomeScan:
         items = []
         for path in self.inputs:
             data, sel = self.read(path)
-            plan = windows.make_plan(data, **self.kw)
-            t, lo, hi, gap = plan.arrays()
-            items.append((data, sel, plan, t, lo, hi, gap, np.flatnonzero(~gap)))
+            plan, t, lo, hi, gap, keep, skip = self._plan(path, data)
+            items.append((data, sel, plan, t, lo, hi, gap, keep, skip, np.flatnonzero(~skip)))
         setup = None
         if self.null is not None:           # prepared now, scanned after the genome (the process group is kept)
             setup = null_mod.NullSetup(self.null, items[0][0], self.neutral, items[0][1], self.grids, **self.kw)
         A = np.array([float(v) for v in GridOrder(self.grids).A])
-        seqs = [(d.genPos, A, t[live], lo[live], hi[live], None) for d, _, _, t, lo, hi, _, live in items]
+        # an input with no centre here is in no rank's range, so it is never loaded (sharding.pieces)
+        seqs = [(d.genPos, A, t[live], lo[live], hi[live], None) for d, _, _, t, lo, hi, _, _, _, live in items]
 
         def open_dev(i):
             return DeviceScan(items[i][0], self.neutral, items[i][1], self.grids, device=device)
@@ -614,14 +685,15 @@ class GenomeScan:
               f'in {dt:.3f} s')
         order = GridOrder(self.grids)
         o = 0
-        for i, (data, sel, plan, t, lo, hi, gap, live) in enumerate(items):
+        for i, (data, sel, plan, t, lo, hi, gap, keep, skip, live) in enumerate(items):
             rows = empty_rows(len(plan))
             if got is not None:
                 for col, v in zip(rows, got):
                     col[live] = v[o:o + len(live)]
             o += len(live)
-            write_scan(self.files['out'][i], plan, order, *rows)
+            wplan, (_, _, _, wgap), wrows, _ = select_rows(keep, plan, (t, lo, hi, gap), rows, None)
+            write_scan(self.files['out'][i], wplan, order, *wrows)
             if null_T is not None:
-                write_pvalues(self.files['pvalues'][i], plan, order, rows, gap, null_T)
-            self._add_regions(self.inputs[i], plan, order, rows, gap)
+                write_pvalues(self.files['pvalues'][i], wplan, order, wrows, wgap, null_T)
+            self._add_regions(self.inputs[i], plan, order, rows, skip)
             print(f'{os.path.basename(self.inputs[i])}: {len(plan)} rows, written to {self.files["out"][i]}')

@@ -26,12 +26,13 @@ class ScanPlan:
         self._f0 = []        # first output column (physPos) as text
         self._f1 = []        # second output column (genPos) as text
         self.gap = []        # --noCenter gap rows (already complete in f0)
+        self._pos = []       # --noCenter: the numeric midpoint of every row (f0 and gap lines hold it as text)
         self.site_phys = None
         self.site_gen = None
 
-    def add(self, t, lo, hi, f0, f1):
+    def add(self, t, lo, hi, f0, f1, pos=None):
         self.t.append(t); self.lo.append(lo); self.hi.append(hi)
-        self._f0.append(f0); self._f1.append(f1); self.gap.append(False)
+        self._f0.append(f0); self._f1.append(f1); self.gap.append(False); self._pos.append(pos)
 
     def set_sites(self, data, idx):
         """All rows are centred on the sites `idx` (a numpy index array)."""
@@ -56,9 +57,26 @@ class ScanPlan:
             return f'{self.site_phys[j]}', f'{self.site_gen[j]}'
         return self._f0[j], self._f1[j]
 
-    def add_gap(self, line):
+    def add_gap(self, line, pos=None):
         self.t.append(0.); self.lo.append(0); self.hi.append(-1)
-        self._f0.append(line); self._f1.append(''); self.gap.append(True)
+        self._f0.append(line); self._f1.append(''); self.gap.append(True); self._pos.append(pos)
+
+    def phys(self):
+        """float64 [rows]: the physPos of every row as a number (the site's position, or the --noCenter midpoint,
+        gap rows included)."""
+        if self.site_phys is not None:
+            return self.site_phys.astype(np.float64)
+        return np.array(self._pos, dtype=np.float64)
+
+    def take(self, idx):
+        """A plan of the rows ``idx`` (ascending indices) only, in that order."""
+        sub = ScanPlan()
+        sub.t, sub.lo, sub.hi, sub.gap = (np.asarray(a)[idx] for a in (self.t, self.lo, self.hi, self.gap))
+        if self.site_phys is not None:
+            sub.site_phys, sub.site_gen = self.site_phys[idx], self.site_gen[idx]
+        else:
+            sub._f0, sub._f1, sub._pos = ([v[i] for i in idx] for v in (self._f0, self._f1, self._pos))
+        return sub
 
     def arrays(self):
         return (np.array(self.t, dtype=np.float64), np.array(self.lo, dtype=np.int64),
@@ -174,9 +192,9 @@ def plan_fixsize_no_center(data, w, s):
             ei += 1
         gen_site = midpos * data.Rrate
         if si >= ei:
-            plan.add_gap('%d\t%g\t0\tNA\tNA\tNA\t0\n' % (midpos, gen_site))
+            plan.add_gap('%d\t%g\t0\tNA\tNA\tNA\t0\n' % (midpos, gen_site), midpos)
         else:
-            plan.add(gen_site, si, ei, f'{midpos}', f'{midpos * data.Rrate}')
+            plan.add(gen_site, si, ei, f'{midpos}', f'{midpos * data.Rrate}', midpos)
         start += s; midpos += s; end += s
     return plan
 
