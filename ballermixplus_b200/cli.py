@@ -7,8 +7,9 @@ GPU, ``--support`` / ``--supportDrop`` write support intervals of A_hat, x_hat a
 / ``--refineSteps`` write the rows again at the best point of a finer grid around each maximum (refine.py),
 ``--inputList`` scans one input per chromosome in one run (scan.GenomeScan), and ``--regions`` / ``--threshold``
 write one line per run of rows above a CLR cut, with its peak, a support interval for the target's position and,
-with ``--null``, a region p-value (regions.py), and ``--targets`` scans only the rows whose centre lies in listed
-intervals, every output a line-for-line subset of the full scan's (targets.py).
+with ``--null``, a region p-value (regions.py), ``--targets`` scans only the rows whose centre lies in listed
+intervals, every output a line-for-line subset of the full scan's (targets.py), and ``--balPos`` writes each row's
+maximum over the alpha >= 1 and the alpha < 1 half of the grid from the same scan (balpos.py).
 Differences, all on paths where the reference raises (SURVEY.md appendix A.2,
 DESIGN.md "flags without a reference behaviour"): ``--rangeA``, ``--findPos`` and
 ``--minCount`` with ``--noFreq`` work here.
@@ -18,6 +19,7 @@ import os
 import sys
 from datetime import datetime
 
+from .balpos import check_grid
 from .grids import Grids
 from .helpers import getConfig, getSpect
 from .inputs import InputData
@@ -134,6 +136,18 @@ def build_parser():
                         'is the exception: a row that is not kept ends a region and stops a '
                         'position interval, as a gap row does, so a region or interval that reaches the first or last '
                         'kept row of a target is cut there. The --null replicates are still scanned in full.')
+    p.add_argument('--balPos', dest='balPos', default=None,
+                   help='Also write FILE: per output row, the row\'s maximum over the balancing half of the grid (alpha '
+                        '>= 1: CLR_bal, x_bal, s_bal, A_bal, nSites_bal) and over the sweep half (alpha < 1: CLR_pos '
+                        '...), each by the reference\'s rule restricted to its points and printed as the output prints '
+                        'its row; max(CLR_bal, CLR_pos) is the row\'s CLR. Both come from the same scan as the output. '
+                        'Each half keeps this run\'s A and x grids: with the default x grid the bal half is the '
+                        '--findBal grid, but the pos half is not the --findPos statistic, which also changes the x grid '
+                        '(0.1..0.9). CLR_bal - CLR_pos is a difference of composite-likelihood maxima that ranks how '
+                        'clearly a row prefers one half; it is not a calibrated test. Needs alpha values on both sides '
+                        'of 1 (not --fixAlpha, --findBal or --findPos). With --inputList: an existing directory, input '
+                        'chr7.txt writes DIR/chr7.txt. With --support the halves take a second scan. Works under '
+                        'torchrun; no other output changes.')
     return p
 
 
@@ -183,6 +197,9 @@ def main(argv=None):
     if opt.regions is not None and opt.threshold is None and opt.null is None:
         parser.error(REGIONS_NEED_A_CUT)
 
+    if opt.balPos is not None:
+        _check_balpos(parser, opt)
+
     inputs = opt.infile
     if opt.inputList:
         inputs = _check_list_mode(parser, opt)
@@ -223,7 +240,7 @@ def main(argv=None):
          phys=opt.phys, noCenter=opt.noCenter, device=opt.device, support=opt.support,
          support_drop=opt.supportDrop, null=opt.null, pvalues=opt.pvalues, refine=opt.refine,
          refine_steps=opt.refineSteps, regions=opt.regions, threshold=opt.threshold,
-         input_name=os.path.basename(opt.infile), targets=targets)
+         input_name=os.path.basename(opt.infile), targets=targets, balpos=opt.balPos)
     print(f'\n{datetime.now()}. Pipeline finished.')
 
 
@@ -239,17 +256,36 @@ def _check_list_mode(parser, opt):
     if opt.outfile is None:
         parser.error('--inputList needs -o DIR')
     for flag, d in (('-o', opt.outfile), ('--support', opt.support), ('--pvalues', opt.pvalues),
-                    ('--refine', opt.refine)):
+                    ('--refine', opt.refine), ('--balPos', opt.balPos)):
         if d is not None and not os.path.isdir(d):
             parser.error(f'--inputList: {flag} {d} is not an existing directory')
     try:
-        files = list_outputs(inputs, out=opt.outfile, support=opt.support, pvalues=opt.pvalues, refine=opt.refine)
+        files = list_outputs(inputs, out=opt.outfile, support=opt.support, pvalues=opt.pvalues, refine=opt.refine,
+                             balpos=opt.balPos)
         if opt.regions is not None:
             reads = [opt.infile, opt.spectfile] + ([opt.null] + read_list(opt.null) if opt.null else [])
             check_regions_file(opt.regions, inputs, files, reads)
     except ValueError as exc:
         parser.error(str(exc))
     return inputs
+
+
+def _check_balpos(parser, opt):
+    """``--balPos``: refused before any input is read with --getSpect or --getConfig, for a grid with no alpha on
+    one side of 1, and (one input) for a file the run reads or writes; --inputList checks its directory with the
+    other output directories (``_check_list_mode``)."""
+    if opt.getSpec or opt.getConfig:
+        parser.error('--balPos writes rows of a scan; --getSpect and --getConfig do not scan')
+    try:
+        check_grid(Grids(opt.x, opt.abeta, opt.bal, opt.pos, opt.seqA, opt.listA).abeta)
+    except ValueError as exc:
+        parser.error(str(exc))
+    if opt.inputList:
+        return
+    others = [opt.infile, opt.spectfile, opt.outfile, opt.support, opt.pvalues, opt.refine, opt.regions, opt.targets,
+              opt.null] + (read_list(opt.null) if opt.null else [])
+    if names_one_of(opt.balPos, others):
+        parser.error(f'--balPos {opt.balPos} is a file this run reads or writes')
 
 
 def _check_targets(parser, opt, inputs):
@@ -261,11 +297,12 @@ def _check_targets(parser, opt, inputs):
         parser.error('--targets selects the rows of a scan; --getSpect and --getConfig do not scan')
     if opt.inputList:
         names = [os.path.basename(p) for p in inputs]
-        files = list_outputs(inputs, out=opt.outfile, support=opt.support, pvalues=opt.pvalues, refine=opt.refine)
+        files = list_outputs(inputs, out=opt.outfile, support=opt.support, pvalues=opt.pvalues, refine=opt.refine,
+                             balpos=opt.balPos)
         written = [f for fs in files.values() for f in fs] + [opt.regions]
     else:
         names = [os.path.basename(opt.infile)]
-        written = [opt.outfile, opt.support, opt.pvalues, opt.refine, opt.regions]
+        written = [opt.outfile, opt.support, opt.pvalues, opt.refine, opt.regions, opt.balPos]
     if names_one_of(opt.targets, written):
         parser.error(f'--targets {opt.targets} is a file this run writes')
     try:
@@ -293,7 +330,7 @@ def _main_list(opt, inputs, targets=None):
     GenomeScan(inputs, read, Neutral, grid, opt.outfile, fixSize=opt.size, r=opt.w, s=opt.step, phys=opt.phys,
                noCenter=opt.noCenter, device=opt.device, support=opt.support, support_drop=opt.supportDrop,
                null=opt.null, pvalues=opt.pvalues, refine=opt.refine, refine_steps=opt.refineSteps,
-               regions=opt.regions, threshold=opt.threshold, targets=targets)
+               regions=opt.regions, threshold=opt.threshold, targets=targets, balpos=opt.balPos)
     print(f'\n{datetime.now()}. Pipeline finished.')
 
 

@@ -18,7 +18,7 @@ ABI_SYMBOLS = (
     'blmx_load', 'blmx_scan', 'blmx_scan_device', 'blmx_scan_oneshot', 'blmx_set_option',
     'blmx_last_counters', 'blmx_last_counters6', 'blmx_last_counters8', 'blmx_last_counters9', 'blmx_problem_info',
     'blmx_last_kernel_ms', 'blmx_measure_fp64_peak', 'blmx_scan_profile', 'blmx_scan_surface',
-    'blmx_load_segmented', 'blmx_load_refine', 'blmx_refine',
+    'blmx_load_segmented', 'blmx_load_refine', 'blmx_refine', 'blmx_scan_split', 'blmx_scan_split_device',
 )
 
 
@@ -61,6 +61,10 @@ def lib():
                                 C.POINTER(Result)]
         L.blmx_scan_profile.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.POINTER(Result), C.POINTER(Profile)]
+        L.blmx_scan_split.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.POINTER(Result), C.POINTER(Result * 2)]
+        L.blmx_scan_split_device.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.POINTER(Result), C.POINTER(Result * 2), C.c_void_p]
         L.blmx_scan_surface.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.c_void_p, C.c_void_p]
         L.blmx_scan_device.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
@@ -203,6 +207,24 @@ class Scanner:
         _check(lib().blmx_scan_profile(self._h, n, _ptr(t), _ptr(lo), _ptr(hi), C.byref(res), C.byref(prof)))
         return T, iA, ix, ia, ns, TA, Tx, Ta, nsA
 
+    def scan_split(self, t, lo, hi, half_of_a):
+        """``scan`` plus the rows of each half of the grid (blmx_scan_split); ``half_of_a`` [n_a]: 0 or 1 per alpha
+        in visiting order -> (rows, half 0 rows, half 1 rows), each (T, iA, ix, ia, nsites)."""
+        t, lo, hi = self._centres(t, lo, hi)
+        half = self._halves(half_of_a)
+        n = len(t)
+        rows = [(np.zeros(n, np.float64), *(np.full(n, -1, np.int32) for _ in range(4))) for _ in range(3)]
+        res = [Result(*(_ptr(a) for a in r)) for r in rows]
+        _check(lib().blmx_scan_split(self._h, n, _ptr(t), _ptr(lo), _ptr(hi), _ptr(half), C.byref(res[0]),
+                                     C.byref((Result * 2)(res[1], res[2]))))
+        return tuple(rows)
+
+    def _halves(self, half_of_a):
+        half = np.ascontiguousarray(half_of_a, dtype=np.int8)
+        if half.shape != (self._grid()[2],):
+            raise ValueError('half_of_a must have one entry per alpha')
+        return half
+
     def scan_surface(self, t, lo, hi):
         """The whole likelihood surface (blmx_scan_surface) -> (S [n, n_A, n_x, n_a], nsA [n, n_A]).
         S is T at every grid point; -inf everywhere for an A without sites.  n * n_A * n_x * n_a doubles come
@@ -247,6 +269,14 @@ class Scanner:
         res = Result(d_T, d_iA, d_ix, d_ia, d_ns)
         _check(lib().blmx_scan_device(self._h, int(n), d_t, d_lo, d_hi, C.byref(res),
                                       C.c_void_p(stream)))
+
+    def scan_split_device(self, n, d_t, d_lo, d_hi, half_of_a, out, halves, stream=0):
+        """``scan_split`` with raw DEVICE pointers (ints) in and out, asynchronous on `stream`: ``out`` and each of
+        the two ``halves`` are five pointers (T, iA, ix, ia, nsites); ``half_of_a`` stays a host array."""
+        half = self._halves(half_of_a)
+        hs = (Result * 2)(Result(*halves[0]), Result(*halves[1]))
+        _check(lib().blmx_scan_split_device(self._h, int(n), d_t, d_lo, d_hi, _ptr(half), C.byref(Result(*out)),
+                                            C.byref(hs), C.c_void_p(stream)))
 
     def counters(self):
         """(site pairs, launches) of the most recent scan."""

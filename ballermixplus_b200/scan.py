@@ -13,8 +13,8 @@ from datetime import datetime
 
 import numpy as np
 
-from . import fastio, null as null_mod, refine as refine_mod, regions as regions_mod, support as support_mod, windows
-from . import targets as targets_mod
+from . import balpos as balpos_mod, fastio, null as null_mod, refine as refine_mod, regions as regions_mod
+from . import support as support_mod, targets as targets_mod, windows
 from .native import Scanner
 from .problem import GridOrder, build_problem
 
@@ -76,6 +76,30 @@ class DeviceScan:
                                  *[x.data_ptr() for x in idx], stream=torch.cuda.current_stream(device).cuda_stream)
         self._keep = (d_t, d_lo, d_hi)              # inputs stay alive until the stream has consumed them
         return (T, *idx)
+
+    def run_split(self, t, lo, hi):
+        """``run`` plus the rows of the balancing (alpha >= 1) and the sweep (alpha < 1) half of the grid, from one
+        scan (blmx_scan_split, balpos.py) -> (rows, bal rows, pos rows), each (T, iA, ix, ia, nsites)."""
+        return self.scanner.scan_split(t, lo, hi, balpos_mod.half_of_a(self.order.a))
+
+    def run_split_device(self, t, lo, hi, torch, device):
+        """``run_split`` with the results left on the device, as ``run_device`` -> 15 tensors: the rows, then the
+        bal rows, then the pos rows, each (T float64, iA, ix, ia, nsites int32)."""
+        n = len(t)
+        d_t = torch.from_numpy(np.ascontiguousarray(t, dtype=np.float64)).to(device)
+        d_lo = torch.from_numpy(np.ascontiguousarray(lo, dtype=np.int64)).to(device)
+        d_hi = torch.from_numpy(np.ascontiguousarray(hi, dtype=np.int64)).to(device)
+        out = []
+        for _ in range(3):
+            idx = [torch.full((n,), -1, dtype=torch.int32, device=device) for _ in range(4)]
+            idx[3].zero_()
+            out.append((torch.zeros(n, dtype=torch.float64, device=device), *idx))
+        ptrs = [tuple(x.data_ptr() for x in rows) for rows in out]
+        self.scanner.scan_split_device(n, d_t.data_ptr(), d_lo.data_ptr(), d_hi.data_ptr(),
+                                       balpos_mod.half_of_a(self.order.a), ptrs[0], ptrs[1:],
+                                       stream=torch.cuda.current_stream(device).cuda_stream)
+        self._keep = (d_t, d_lo, d_hi)
+        return tuple(x for rows in out for x in rows)
 
     def decode(self, T, iA, ix, ia, ns):
         return self.order.decode(T, iA, ix, ia, ns)
@@ -174,23 +198,26 @@ def ranks_own_a_gpu():
     return device_count() >= _local_world()
 
 
-def scan_rows_multi_gpu(dev, t, lo, hi, rank, world, local_rank, keep_group=False):
+def scan_rows_multi_gpu(dev, t, lo, hi, rank, world, local_rank, keep_group=False, split=False):
     """One process per GPU (torchrun): every rank scans a cost-balanced contiguous slice of the centres,
     one gather brings the rows to rank 0 (sharding.py).  When every rank of the node has its own GPU the rows
     stay on the device from the scan kernel to the NCCL gather (``DeviceScan.run_device``); when several ranks
     share one device (tests on a one-GPU box) the gather runs over gloo on host tensors.  Returns the five
     result arrays on rank 0 and None elsewhere.  ``keep_group``: leave the process group this call starts
-    running for a later scan (``end_group`` ends it)."""
+    running for a later scan (``end_group`` ends it).  ``split`` (``--balPos``): the scan is ``run_split`` and 15
+    arrays come back, the rows and then the bal and the pos rows."""
     seq = (dev.problem.genpos, dev.problem.A, t, lo, hi, getattr(dev.problem, 'seg_start', None))
-    return scan_seqs_multi_gpu([seq], lambda i: dev, dev.scanner.device, rank, world, keep_group=keep_group)
+    return scan_seqs_multi_gpu([seq], lambda i: dev, dev.scanner.device, rank, world, keep_group=keep_group,
+                               split=split)
 
 
-def scan_seqs_multi_gpu(seqs, open_dev, device, rank, world, keep_group=False, release=False):
+def scan_seqs_multi_gpu(seqs, open_dev, device, rank, world, keep_group=False, release=False, split=False):
     """``scan_rows_multi_gpu`` over several sequences (sharding.scan_sharded_seqs): the centres of all of them are
     cut into cost-balanced ranges, and a rank scans only the sequences its range touches, on the DeviceScan
     ``open_dev(i)`` gives for sequence i.  ``seqs``: one (genpos, A, t, lo, hi, seg_start) per sequence.
     ``release``: close each DeviceScan once its rows are computed, so that one sequence at a time is resident.
-    Returns the five result arrays of the concatenated centre list on rank 0 and None elsewhere."""
+    Returns the five result arrays of the concatenated centre list on rank 0 and None elsewhere (with ``split``:
+    the 15 of ``run_split``, gathered in one wider block, sharding.pack_split_rows)."""
     import torch
     import torch.distributed as dist
     from . import sharding
@@ -212,10 +239,12 @@ def scan_seqs_multi_gpu(seqs, open_dev, device, rank, world, keep_group=False, r
         dev = open_dev(i)
         try:
             if own_gpu:
-                got = dev.run_device(ts, los, his, torch, where)
+                got = (dev.run_split_device if split else dev.run_device)(ts, los, his, torch, where)
                 if release:             # the rows stay on the device; the handle may go once they are written
                     torch.cuda.current_stream(where).synchronize()
                 return got
+            if split:
+                return tuple(torch.from_numpy(np.ascontiguousarray(a)) for r in dev.run_split(ts, los, his) for a in r)
             return tuple(torch.from_numpy(np.ascontiguousarray(a)) for a in dev.run(ts, los, his))
         finally:
             if release:
@@ -223,7 +252,7 @@ def scan_seqs_multi_gpu(seqs, open_dev, device, rank, world, keep_group=False, r
 
     ok = False
     try:
-        got = sharding.scan_sharded_seqs(seqs, rank, world, scan_fn, dist, torch, device=where)
+        got = sharding.scan_sharded_seqs(seqs, rank, world, scan_fn, dist, torch, device=where, split=split)
         ok = True
         return None if got is None else tuple(a.cpu().numpy() for a in got)
     finally:
@@ -269,8 +298,12 @@ def empty_rows(n):
     return (np.zeros(n), *(np.full(n, -1, np.int32) for _ in range(3)), np.zeros(n, np.int32))
 
 
-def check_options(world, support, support_drop, refine, refine_steps, null, pvalues, regions=None, threshold=None):
-    """Refuse option combinations before any work -> (support_drop, refine_steps, threshold), checked."""
+def check_options(world, support, support_drop, refine, refine_steps, null, pvalues, regions=None, threshold=None,
+                  balpos=None, grids=None):
+    """Refuse option combinations before any work -> (support_drop, refine_steps, threshold), checked.  ``balpos``
+    needs alpha values of ``grids`` on both sides of 1."""
+    if balpos is not None:
+        balpos_mod.check_grid(grids.abeta)
     if support is not None or regions is not None:
         support_drop = support_mod.check_drop(support_drop)
     if support is not None and world > 1:
@@ -303,22 +336,32 @@ def open_outputs(*paths):
                 pass
 
 
-def scan_plan(dev, t, lo, hi, gap, support_drop=None):
+def scan_plan(dev, t, lo, hi, gap, support_drop=None, balpos=False):
     """The rows of a plan's arrays on one GPU (gap rows, and rows ``--targets`` skips, passed in ``gap``, left
-    unscanned) and, with ``support_drop``, their support intervals -> (rows, intervals or None)."""
+    unscanned), with ``support_drop`` their support intervals, and with ``balpos`` the rows of the two halves of
+    the grid (``--balPos``) -> (rows, intervals or None, (bal rows, pos rows) or None).  ``--balPos`` alone takes
+    the rows and the halves from one ``run_split``; with ``--support`` the profile scan keeps the rows and a second
+    scan, ``run_split``, gives the halves (DESIGN.md §3.14)."""
     rows = empty_rows(len(t))
     iv = {k: np.full(len(t), -1, np.int32) for k in INTERVAL_KEYS} if support_drop is not None else None
+    halves = (empty_rows(len(t)), empty_rows(len(t))) if balpos else None
     live = np.flatnonzero(~gap)
     if len(live):
+        got_halves = ()
         if support_drop is not None:
             got, got_iv = scan_with_support(dev, t[live], lo[live], hi[live], support_drop)
             for k, v in got_iv.items():
                 iv[k][live] = v
+            if balpos:
+                got_halves = dev.run_split(t[live], lo[live], hi[live])[1:]
+        elif balpos:
+            got, *got_halves = dev.run_split(t[live], lo[live], hi[live])
         else:
             got = dev.run(t[live], lo[live], hi[live])
-        for col, v in zip(rows, got):
-            col[live] = v
-    return rows, iv
+        for dst, src in zip((rows,) + (halves or ()), (got,) + tuple(got_halves)):
+            for col, v in zip(dst, src):
+                col[live] = v
+    return rows, iv, halves
 
 
 def select_rows(keep, plan, arrays, rows, iv):
@@ -330,6 +373,14 @@ def select_rows(keep, plan, arrays, rows, iv):
     idx = np.flatnonzero(keep)
     return (plan.take(idx), tuple(a[idx] for a in arrays), tuple(c[idx] for c in rows),
             None if iv is None else {k: v[idx] for k, v in iv.items()})
+
+
+def kept_halves(keep, halves):
+    """The half rows of ``--balPos`` at the rows ``keep`` selects (as ``select_rows``; None passes through)."""
+    if keep is None or halves is None:
+        return halves
+    idx = np.flatnonzero(keep)
+    return tuple(tuple(c[idx] for c in h) for h in halves)
 
 
 def skipped(gap, keep):
@@ -391,22 +442,26 @@ class Scan:
     ``targets`` (a ``targets.Targets``): scan only the rows whose physPos lies in a target of the input named
     ``input_name``; every file then holds the header and, in order, exactly the lines of the full run at those rows
     (``results`` too holds those rows only).  A row not kept ends a region and stops a position interval, as a gap
-    row does."""
+    row does.
+
+    ``balpos`` (a path): also write, per row of ``outfile``, the row maximum over the balancing (alpha >= 1) and
+    over the sweep (alpha < 1) half of the grid (balpos.py), from the same scan.  Works under torchrun; no other
+    file changes."""
 
     def __init__(self, InputData, NeutralSFS, NormalizedBetaBinom, Grids, outfile, fixSize=False,
                  r=0, s=1, phys=False, noCenter=False, device=0, support=None,
                  support_drop=support_mod.DEFAULT_DROP, null=None, pvalues=None, refine=None,
                  refine_steps=refine_mod.DEFAULT_STEPS, regions=None, threshold=None, input_name=None,
-                 targets=None):
+                 targets=None, balpos=None):
         rank, world, local_rank = _world()
         support_drop, refine_steps, threshold = check_options(world, support, support_drop, refine, refine_steps,
-                                                              null, pvalues, regions, threshold)
+                                                              null, pvalues, regions, threshold, balpos, Grids)
         plan = windows.make_plan(InputData, fixSize=fixSize, r=r, s=s, phys=phys, noCenter=noCenter)
         name = os.path.basename(outfile) if input_name is None else input_name
         keep = None if targets is None else targets.keep(name, plan)
         if rank == 0:
             print('writing output to %s' % (outfile))
-            open_outputs(outfile, support, pvalues, refine, regions)
+            open_outputs(outfile, support, pvalues, refine, regions, balpos)
             if keep is not None:
                 print(targets_mod.kept_line(name, keep))
         setup = None
@@ -426,18 +481,23 @@ class Scan:
             if world > 1:
                 live = np.flatnonzero(~skip)
                 rows, iv = empty_rows(len(plan)), None
+                halves = (empty_rows(len(plan)), empty_rows(len(plan))) if balpos is not None else None
                 if len(live):
                     got = scan_rows_multi_gpu(dev, t[live], lo[live], hi[live], rank, world, local_rank,
-                                              keep_group=setup is not None)
+                                              keep_group=setup is not None, split=balpos is not None)
                     if got is not None:
-                        for col, v in zip(rows, got):
+                        for col, v in zip(rows + sum(halves or (), ()), got):
                             col[live] = v
             else:
-                rows, iv = scan_plan(dev, t, lo, hi, skip, support_drop if support is not None else None)
+                rows, iv, halves = scan_plan(dev, t, lo, hi, skip, support_drop if support is not None else None,
+                                             balpos=balpos is not None)
             wplan, (wt, wlo, whi, wgap), wrows, wiv = select_rows(keep, plan, (t, lo, hi, gap), rows, iv)
             self.results = wrows if rank == 0 else None
             if rank == 0:
                 write_scan(outfile, wplan, dev.order, *wrows)
+                if balpos is not None:
+                    self.halves = kept_halves(keep, halves)
+                    balpos_mod.write_balpos(balpos, wplan, dev.order, *self.halves)
                 if support is not None:
                     self.support = wiv
                     write_support(support, wplan, dev.order, wrows, wiv)
@@ -552,17 +612,21 @@ class GenomeScan:
 
     ``targets`` (a ``targets.Targets``, inputs named by file name): each input keeps only the rows in its targets, as
     in ``Scan``; the centres of the kept rows alone are scanned (and sharded under torchrun), and an input with no
-    kept row to scan is read and planned but never loaded on a GPU."""
+    kept row to scan is read and planned but never loaded on a GPU.
+
+    ``balpos`` (a directory, like ``outdir``): the ``--balPos`` file of every input, as ``Scan`` writes it; on one GPU
+    and under torchrun, where the half rows travel in the same gather as the rows."""
 
     def __init__(self, inputs, read, NeutralSFS, Grids, outdir, fixSize=False, r=0, s=1, phys=False,
                  noCenter=False, device=0, support=None, support_drop=support_mod.DEFAULT_DROP, null=None,
                  pvalues=None, refine=None, refine_steps=refine_mod.DEFAULT_STEPS, regions=None, threshold=None,
-                 targets=None):
+                 targets=None, balpos=None):
         rank, world, local_rank = _world()
         support_drop, refine_steps, threshold = check_options(world, support, support_drop, refine, refine_steps,
-                                                              null, pvalues, regions, threshold)
+                                                              null, pvalues, regions, threshold, balpos, Grids)
         self.inputs = list(inputs)
-        self.files = list_outputs(self.inputs, out=outdir, support=support, pvalues=pvalues, refine=refine)
+        self.files = list_outputs(self.inputs, out=outdir, support=support, pvalues=pvalues, refine=refine,
+                                  balpos=balpos)
         if regions is not None:
             check_regions_file(regions, self.inputs, self.files)
         if rank == 0:
@@ -635,10 +699,13 @@ class GenomeScan:
             else:
                 dev = DeviceScan(data, self.neutral, sel, self.grids, device=device)
             try:
-                rows, iv = scan_plan(dev, t, lo, hi, skip, support_drop if 'support' in self.files else None)
+                rows, iv, halves = scan_plan(dev, t, lo, hi, skip, support_drop if 'support' in self.files else None,
+                                             balpos='balpos' in self.files)
                 dt = time.perf_counter() - t0
                 wplan, (wt, wlo, whi, wgap), wrows, wiv = select_rows(keep, plan, (t, lo, hi, gap), rows, iv)
                 write_scan(self.files['out'][i], wplan, dev.order, *wrows)
+                if halves is not None:
+                    balpos_mod.write_balpos(self.files['balpos'][i], wplan, dev.order, *kept_halves(keep, halves))
                 if wiv is not None:
                     write_support(self.files['support'][i], wplan, dev.order, wrows, wiv)
                 if 'refine' in self.files:
@@ -672,7 +739,7 @@ class GenomeScan:
         got = None
         if sum(len(s[2]) for s in seqs):
             got = scan_seqs_multi_gpu(seqs, open_dev, device, rank, world, keep_group=setup is not None,
-                                      release=True)
+                                      release=True, split='balpos' in self.files)
         dt = time.perf_counter() - t0
         null_T = None
         if setup is not None:
@@ -687,12 +754,15 @@ class GenomeScan:
         o = 0
         for i, (data, sel, plan, t, lo, hi, gap, keep, skip, live) in enumerate(items):
             rows = empty_rows(len(plan))
+            halves = (empty_rows(len(plan)), empty_rows(len(plan))) if 'balpos' in self.files else None
             if got is not None:
-                for col, v in zip(rows, got):
+                for col, v in zip(rows + sum(halves or (), ()), got):
                     col[live] = v[o:o + len(live)]
             o += len(live)
             wplan, (_, _, _, wgap), wrows, _ = select_rows(keep, plan, (t, lo, hi, gap), rows, None)
             write_scan(self.files['out'][i], wplan, order, *wrows)
+            if halves is not None:
+                balpos_mod.write_balpos(self.files['balpos'][i], wplan, order, *kept_halves(keep, halves))
             if null_T is not None:
                 write_pvalues(self.files['pvalues'][i], wplan, order, wrows, wgap, null_T)
             self._add_regions(self.inputs[i], plan, order, rows, skip)

@@ -95,6 +95,16 @@ def unpack_rows(rows, torch):
     return T, rows[:, 2], rows[:, 3], rows[:, 4], rows[:, 5]
 
 
+def pack_split_rows(rows, torch):
+    """The 15 results of a ``--balPos`` scan (the rows, then the bal and the pos rows, five each) as one int32
+    [n, 18] tensor: the rows' six columns of ``pack_rows`` first, then six per half."""
+    return torch.cat([pack_rows(*rows[5 * k:5 * k + 5], torch) for k in range(3)], dim=1)
+
+
+def unpack_split_rows(rows, torch):
+    return tuple(v for k in range(3) for v in unpack_rows(rows[:, 6 * k:6 * k + 6], torch))
+
+
 def gather_rows(rows, counts, rank, world, dist, torch, dst=0):
     """The path's only collective: gather every rank's rows on `dst`, in rank order.
 
@@ -134,7 +144,7 @@ def pieces(offs, b, e):
     return out
 
 
-def scan_sharded_seqs(seqs, rank, world, scan_fn, dist, torch, device=None):
+def scan_sharded_seqs(seqs, rank, world, scan_fn, dist, torch, device=None, split=False):
     """Scan the centres of several sequences (one per chromosome: a genome) on `world` ranks and gather the
     rows on rank 0.
 
@@ -146,21 +156,23 @@ def scan_sharded_seqs(seqs, rank, world, scan_fn, dist, torch, device=None):
     nsites int32) living on that device; it is called once per sequence the rank's range touches, in order,
     and never for the others, so a rank needs only those sequences on its device.  A rank whose range is
     empty sends an empty block made on ``device``.  Returns the five gathered tensors on rank 0 (the
-    concatenated centre list, in order) and None elsewhere.
+    concatenated centre list, in order) and None elsewhere.  ``split`` (``--balPos``): `scan_fn` returns the 15
+    tensors of a split scan, packed wider for the same one gather (``pack_split_rows``), and 15 come back.
     """
     costs, offs = genome_costs(seqs)
     parts = partition(costs, world)
     counts = [e - b for b, e in parts]
     blocks = []
+    pack, unpack = (pack_split_rows, unpack_split_rows) if split else (lambda r, tc: pack_rows(*r, tc), unpack_rows)
     for i, lb, le in pieces(offs, *parts[rank]):
         t, lo, hi = (np.asarray(a)[lb:le] for a in seqs[i][2:5])
-        blocks.append(pack_rows(*scan_fn(i, t, lo, hi), torch))
+        blocks.append(pack(scan_fn(i, t, lo, hi), torch))
     if not blocks:
-        rows = torch.zeros((0, 6), dtype=torch.int32, device=device)
+        rows = torch.zeros((0, 18 if split else 6), dtype=torch.int32, device=device)
     else:
         rows = blocks[0] if len(blocks) == 1 else torch.cat(blocks, dim=0)
     got = gather_rows(rows, counts, rank, world, dist, torch)
-    return unpack_rows(got, torch) if got is not None else None
+    return unpack(got, torch) if got is not None else None
 
 
 def scan_sharded(genpos, A, t, lo, hi, rank, world, scan_fn, dist, torch, seg_start=None, device=None):

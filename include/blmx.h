@@ -155,6 +155,24 @@ typedef struct {
 int blmx_scan_profile(blmx_handle *h, int64_t n_centres, const double *t, const int64_t *lo,
                       const int64_t *hi, const blmx_result *out, const blmx_profile *prof);
 
+/*
+ * Balancing-versus-sweep rows (DESIGN.md §3.14): blmx_scan plus the same rule restricted to each of two halves of
+ * the grid.  half_of_a[ia] (HOST array of n_a entries, alpha in visiting order) is 0 for a grid point of the first
+ * half ("bal": alpha >= 1 on the command line) and 1 for the second ("pos": alpha < 1); any other value is
+ * BLMX_ERR_ARG.  `out` gets exactly what blmx_scan writes; halves[k] gets, per centre, the reference's row over
+ * the grid points of half k only: A in visiting order, then (x, a) in visiting order, strict '>' from T = 0
+ * (from -inf with option report_all), an A without sites skipped; the all-zero row when no point of the half
+ * qualifies.  Pruning stays on: an item proved T <= 0 everywhere is T <= 0 in each half.
+ *
+ * blmx_scan_split: HOST buffers, synchronous.  blmx_scan_split_device: t, lo, hi, out and halves are DEVICE buffers
+ * (half_of_a stays a host array), asynchronous on `cuda_stream`, as blmx_scan_device.
+ */
+int blmx_scan_split(blmx_handle *h, int64_t n_centres, const double *t, const int64_t *lo, const int64_t *hi,
+                    const int8_t *half_of_a, const blmx_result *out, const blmx_result *halves /* [2] */);
+int blmx_scan_split_device(blmx_handle *h, int64_t n_centres, const double *d_t, const int64_t *d_lo,
+                           const int64_t *d_hi, const int8_t *half_of_a, const blmx_result *d_out,
+                           const blmx_result *d_halves /* [2] */, void *cuda_stream);
+
 /* The full surface of a few centres (for plots and tests): S[j][iA][ix*n_a + ia], nsA[j][iA]. */
 int blmx_scan_surface(blmx_handle *h, int64_t n_centres, const double *t, const int64_t *lo,
                       const int64_t *hi, double *S, int32_t *nsA);

@@ -3,10 +3,11 @@
     python tools/sass_compare.py OLD.so NEW.so
 
 Every scan_kernel<J, GROUP, FAR> of OLD (the kernel before it took the SURF flag) is compared, instruction
-listing for instruction listing (cuobjdump -sass), with scan_kernel<J, GROUP, FAR, SURF = false> of NEW; a
-kernel OLD already has with the SURF flag is compared with the same instantiation in NEW.  Build both with the
-same nvcc flags.  bound_kernel, which the scan runs before scan_kernel, is compared as well.  Exit status 1 if any
-listing differs.
+listing for instruction listing (cuobjdump -sass), with scan_kernel<J, GROUP, FAR, SURF = false> of NEW, and every
+scan_kernel<J, GROUP, FAR, SURF> of OLD (before the SPLIT flag) with scan_kernel<J, GROUP, FAR, SURF, SPLIT = false>;
+a kernel OLD already has with the SPLIT flag is compared with the same instantiation in NEW.  Build both with the
+same nvcc flags.  bound_kernel, which the scan runs before scan_kernel, and reduce_kernel, which runs after it, are
+compared as well.  Exit status 1 if any listing differs.
 """
 import re
 import subprocess
@@ -34,12 +35,13 @@ def main():
     old, new = scan_kernels(sys.argv[1]), scan_kernels(sys.argv[2])
     same = 0
     for name in sorted(old):
-        twin = name if name.count(',') == 3 else name[:-1] + ', 0>'
+        twin = name[:-1] + ', 0' * (4 - name.count(',')) + '>'
         ok = old[name] == new.get(twin)
         same += ok
         print(f'{"identical" if ok else "DIFFERENT"}  {name} -> {twin}  ({len(old[name].splitlines())} lines)')
     print(f'{same}/{len(old)} identical')
-    old_b, new_b = scan_kernels(sys.argv[1], 'bound_kernel('), scan_kernels(sys.argv[2], 'bound_kernel(')
+    old_b, new_b = ({**scan_kernels(so, 'bound_kernel('), **scan_kernels(so, 'reduce_kernel(')}
+                    for so in sys.argv[1:3])
     same_b = sum(old_b[k] == new_b.get(k) for k in old_b)
     for k in sorted(old_b):
         print(f'{"identical" if old_b[k] == new_b.get(k) else "DIFFERENT"}  {k}  ({len(old_b[k].splitlines())} lines)')
