@@ -33,7 +33,9 @@
 typedef struct { double s, c; } ksum;               /* Neumaier compensated accumulator */
 static inline void ksum_add(ksum *k, double v) {
     double t = k->s + v;
-    if (fabs(k->s) >= fabs(v)) k->c += (k->s - t) + v; else k->c += (v - t) + k->s;
+    if (isfinite(t)) {                              /* an inf or nan sum is the sum: log(0) = -inf stays -inf */
+        if (fabs(k->s) >= fabs(v)) k->c += (k->s - t) + v; else k->c += (v - t) + k->s;
+    }
     k->s = t;
 }
 

@@ -51,13 +51,17 @@ def _check_split(prob, t, lo, hi, half, report_all=0, **opts):
     S, nsA = surface_oracle.problem_surface(prob, t, lo, hi)
     for h, got in ((0, bal), (1, pos)):
         want = _half_rows(S, nsA, half, h, bool(report_all))
-        err = np.abs(got[0] - want[0]) / np.maximum(np.abs(want[0]), 1.)
-        assert err.max() <= 1e-9, err.max()
+        fin = np.isfinite(want[0])                      # T = +inf (a class with G = 0) must be +inf
+        assert np.array_equal(got[0][~fin], want[0][~fin])
+        err = np.abs(got[0][fin] - want[0][fin]) / np.maximum(np.abs(want[0][fin]), 1.)
+        assert err.size == 0 or err.max() <= 1e-9, err.max()
         for g, w in zip(got[1:], want[1:]):
             assert np.array_equal(g, w)
-    # every row's CLR is the better half's (report_all: both halves start from -inf as the row does)
-    best = np.where(bal[0] >= pos[0], bal[0], pos[0])
-    assert np.array_equal(best, rows[0])
+    # every row's CLR is the better half's (report_all: both halves start from -inf as the row does); a half that
+    # reports no grid point (iA = -1, T = 0: no alpha in it, or nothing above the floor) takes no part
+    best = np.maximum(np.where(bal[1] >= 0, bal[0], -np.inf), np.where(pos[1] >= 0, pos[0], -np.inf))
+    assert np.array_equal(np.where(rows[1] >= 0, best, 0.0), rows[0])
+    assert np.array_equal(rows[1] >= 0, (bal[1] >= 0) | (pos[1] >= 0))
     return bal, pos
 
 
