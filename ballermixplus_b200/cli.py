@@ -9,7 +9,8 @@ GPU, ``--support`` / ``--supportDrop`` write support intervals of A_hat, x_hat a
 write one line per run of rows above a CLR cut, with its peak, a support interval for the target's position and,
 with ``--null``, a region p-value (regions.py), ``--targets`` scans only the rows whose centre lies in listed
 intervals, every output a line-for-line subset of the full scan's (targets.py), and ``--balPos`` writes each row's
-maximum over the alpha >= 1 and the alpha < 1 half of the grid from the same scan (balpos.py).
+maximum over the alpha >= 1 and the alpha < 1 half of the grid from the same scan (balpos.py), and ``--spectBins`` /
+``--binMap`` give each site the neutral spectrum of its bin (bins.py).
 Differences, all on paths where the reference raises (SURVEY.md appendix A.2,
 DESIGN.md "flags without a reference behaviour"): ``--rangeA``, ``--findPos`` and
 ``--minCount`` with ``--noFreq`` work here.
@@ -20,8 +21,9 @@ import sys
 from datetime import datetime
 
 from .balpos import check_grid
+from .bins import BinnedNeutral, attach, read_bin_map, read_spect_bins
 from .grids import Grids
-from .helpers import getConfig, getSpect
+from .helpers import getConfig, getSpect, getSpectBinned
 from .inputs import InputData
 from .neutral import NeutralSFS
 from .null import read_list
@@ -148,6 +150,19 @@ def build_parser():
                         'of 1 (not --fixAlpha, --findBal or --findPos). With --inputList: an existing directory, input '
                         'chr7.txt writes DIR/chr7.txt. With --support the halves take a second scan. Works under '
                         'torchrun; no other output changes.')
+    p.add_argument('--spectBins', dest='spectBins', default=None,
+                   help='With --binMap: text file with one bin per line, "label path", path (relative to the list) a '
+                        'spectrum or configuration file read as --spect is; blank and # lines skipped.')
+    p.add_argument('--binMap', dest='binMap', default=None,
+                   help='With --spectBins: one interval per line, "name start end label", name the input\'s file name '
+                        '(with --inputList, of a listed input; or of a --null replicate), start and end inclusive physPos '
+                        'values; blank and # lines, a header line starting with "input" and fields after the fourth are '
+                        'skipped.  A site covered by an interval takes the neutral spectrum of its label (g and the '
+                        'sample-size proportion of its k and n in that file), every other site --spect; two overlapping '
+                        'intervals of one input with different labels are refused.  With --getSpect or --getConfig '
+                        '(no --spectBins needed): write --spect from the sites no interval covers and --spect.LABEL from '
+                        'the sites of each label, each only when it has sites (no --spect file when the map covers '
+                        'every site).')
     return p
 
 
@@ -204,7 +219,12 @@ def main(argv=None):
     if opt.inputList:
         inputs = _check_list_mode(parser, opt)
     targets = _check_targets(parser, opt, inputs)
+    binned = _check_bins(parser, opt, inputs)
 
+    if (opt.getSpec or opt.getConfig) and binned is not None:
+        print('You\'ve chosen to generate binned helper files...')
+        getSpectBinned(inputs, opt.spectfile, opt.MAF, opt.nosub, binned, config=opt.getConfig)
+        sys.exit()
     if opt.getSpec:
         print('You\'ve chosen to generate site frequency spectrum...')
         print('Concatenated input: %s \nSpectrum file: %s' % (opt.infile, opt.spectfile))
@@ -216,13 +236,14 @@ def main(argv=None):
         getConfig(inputs, opt.spectfile)
         sys.exit()
     if opt.inputList:
-        _main_list(opt, inputs, targets)
+        _main_list(opt, inputs, targets, binned)
         return
 
     print(f'\n{datetime.now()}. Reading input from {opt.infile}')
     data = InputData(opt.infile, opt.nofreq, opt.MAF, opt.nosub, opt.minCount, phys=opt.phys,
                      Rrate=opt.Rrate)
-    Neutral = NeutralSFS(opt.spectfile, opt.nofreq, opt.MAF, opt.nosub)
+    Neutral = _neutral(opt, binned)
+    attach(data, Neutral, os.path.basename(opt.infile))
 
     print(f'\n{datetime.now()}. Initializing...')
     print('Retrieving per-site neutral probabilities...')
@@ -311,10 +332,73 @@ def _check_targets(parser, opt, inputs):
         parser.error(str(exc))
 
 
-def _main_list(opt, inputs, targets=None):
+def _check_bins(parser, opt, inputs):
+    """``--spectBins`` / ``--binMap``: the parsed map (None without them), refused before any input is read when
+    one comes without the other (with --getSpect/--getConfig only the map is needed), when the run writes either
+    file and when either is bad (bins.read_spect_bins, bins.read_bin_map).  Keeps the list's bins in opt._bins."""
+    helper = opt.getSpec or opt.getConfig
+    if opt.binMap is None:
+        if opt.spectBins is not None:
+            parser.error('--spectBins needs --binMap')
+        return None
+    if opt.spectBins is None and not helper:
+        parser.error('--binMap needs --spectBins')
+    if opt.inputList:
+        names = [os.path.basename(p) for p in inputs]
+        written = [] if helper else [f for fs in list_outputs(inputs, out=opt.outfile, support=opt.support,
+                                                               pvalues=opt.pvalues, refine=opt.refine,
+                                                               balpos=opt.balPos).values() for f in fs]
+        written.append(opt.regions)
+    else:
+        names = [os.path.basename(opt.infile)]
+        written = [opt.outfile, opt.support, opt.pvalues, opt.refine, opt.regions, opt.balPos]
+    if opt.null is not None:
+        names += [os.path.basename(p) for p in read_list(opt.null)]
+    try:
+        bins = read_spect_bins(opt.spectBins) if opt.spectBins is not None else []
+        labels = _map_labels(opt.binMap) if helper and opt.spectBins is None else [label for label, _ in bins]
+        if helper:
+            written += [opt.spectfile] + [f'{opt.spectfile}.{label}' for label in labels]
+        for flag, path in (('--spectBins', opt.spectBins), ('--binMap', opt.binMap)):
+            if path is not None and names_one_of(path, written):
+                raise ValueError(f'{flag} {path} is a file this run writes')
+        for label, path in bins:                # --getSpect/--getConfig would overwrite a listed spectrum
+            if names_one_of(path, written):
+                raise ValueError(f'--spectBins {opt.spectBins}: the spectrum {path} of bin {label} is a file this '
+                                 f'run writes')
+        binmap = read_bin_map(opt.binMap, names, labels)
+    except ValueError as exc:
+        parser.error(str(exc))
+    opt._bins = bins
+    return binmap
+
+
+def _map_labels(path):
+    """The labels a --binMap file names, in order of first use (--getSpect/--getConfig without --spectBins)."""
+    labels = []
+    try:
+        with open(path) as fh:
+            for line in fh:
+                f = line.split()
+                if len(f) >= 4 and not f[0].startswith('#') and f[0] != 'input' and f[3] not in labels:
+                    labels.append(f[3])
+    except (OSError, UnicodeDecodeError):
+        pass                                    # read_bin_map reports it
+    return labels
+
+
+def _neutral(opt, binned):
+    """The run's neutral model: NeutralSFS of --spect, or with a bin map the BinnedNeutral of --spect and the
+    --spectBins files."""
+    if binned is None:
+        return NeutralSFS(opt.spectfile, opt.nofreq, opt.MAF, opt.nosub)
+    return BinnedNeutral.read(opt.spectfile, opt._bins, binned, opt.nofreq, opt.MAF, opt.nosub)
+
+
+def _main_list(opt, inputs, targets=None, binned=None):
     """One run over every listed input (scan.GenomeScan), each read and tabulated as the one-input run reads it."""
     print(f'\n{datetime.now()}. {len(inputs)} inputs listed in {opt.infile}')
-    Neutral = NeutralSFS(opt.spectfile, opt.nofreq, opt.MAF, opt.nosub)
+    Neutral = _neutral(opt, binned)
     grid = Grids(opt.x, opt.abeta, opt.bal, opt.pos, opt.seqA, opt.listA)
     print('\nOptimizing over x= ' + ', '.join(['%g' % (x) for x in grid.x]))
     print('\n \t alpha= ' + ', '.join([str(a) for a in grid.abeta]))
@@ -323,6 +407,7 @@ def _main_list(opt, inputs, targets=None):
     def read(path):
         print(f'\n{datetime.now()}. Reading input from {path}')
         data = InputData(path, opt.nofreq, opt.MAF, opt.nosub, opt.minCount, phys=opt.phys, Rrate=opt.Rrate)
+        attach(data, Neutral, os.path.basename(path))
         Neutral.get_neut_probs(data)
         return data, NormalizedBetaBinom(data, grid, opt.nofreq, opt.MAF, opt.nosub)
 

@@ -23,6 +23,7 @@ import sys
 import numpy as np
 
 from . import fastio
+from .inputs import read_site_table
 
 
 def _read_xn(infile):
@@ -47,6 +48,10 @@ def _read_xn(infile):
 
 def getConfig(infile, configfile):
     x, n = _read_xn(infile)
+    _write_config(x, n, configfile)
+
+
+def _write_config(x, n, configfile):
     zero = x == 0
     for _ in range(int(zero.sum())):
         print('Please make sure the input has derived allele frequency. Sites with 0 observed '
@@ -64,6 +69,40 @@ def getConfig(infile, configfile):
 
 def getSpect(infile, spectfile, MAF, nosub):
     x, n = _read_xn(infile)
+    _write_spect(x, n, spectfile, MAF, nosub)
+
+
+def _bin_sites(infile, binmap):
+    """(x, n, bin) of every site of `infile` (or of a list of paths), each site's bin from ``binmap``
+    (bins.BinMap) at its physPos: the first column read as the input reader reads it."""
+    paths = [infile] if isinstance(infile, (str, bytes, os.PathLike)) else list(infile)
+    xs, ns, bs = [], [], []
+    for p in paths:
+        x, n = _read_xn(p)
+        pos = read_site_table(p, True, 1.0)[0]
+        xs.append(x); ns.append(n); bs.append(binmap.site_bins(os.path.basename(p), pos))
+    return np.concatenate(xs), np.concatenate(ns), np.concatenate(bs)
+
+
+def getSpectBinned(infile, spectfile, MAF, nosub, binmap, config=False):
+    """--getSpect / --getConfig with --binMap: ``spectfile`` from the sites no interval covers and
+    ``spectfile.label`` for every label, each only when it has sites and each the file getSpect (getConfig) writes
+    for those sites alone -> the files written.  A bin without sites gets no file (it would be empty, which
+    NeutralSFS refuses), so ``spectfile`` is not written when the map covers every site."""
+    x, n, b = _bin_sites(infile, binmap)
+    out = []
+    for k in [k for k in range(len(binmap.labels) + 1) if np.any(b == k)]:
+        path = spectfile if k == 0 else f'{spectfile}.{binmap.labels[k - 1]}'
+        print(f'Bin {binmap.labels[k - 1] if k else "(no interval)"}: {int(np.sum(b == k))} sites -> {path}')
+        if config:
+            _write_config(x[b == k], n[b == k], path)
+        else:
+            _write_spect(x[b == k], n[b == k], path, MAF, nosub)
+        out.append(path)
+    return out
+
+
+def _write_spect(x, n, spectfile, MAF, nosub):
     if MAF:
         over = x > n / 2
         if np.any(over):

@@ -116,7 +116,10 @@ class ScanProblem:
     """Host arrays of one blmx_problem (see include/blmx.h for the meaning of each).
 
     ``seg_start`` (optional): first site of each segment of a problem made of several sequences laid end to
-    end (blmx_load_segmented); ``Scanner.load`` then loads it segmented."""
+    end (blmx_load_segmented); ``Scanner.load`` then loads it segmented.  ``layout``: None, or for a binned
+    problem (problem.build_binned) the (P, sel_class) its SP was built from, which refine.py's fine rows use."""
+
+    layout = None
 
     def __init__(self, genpos, cls, G, SP, A, n_x, n_a, seg_start=None):
         self.seg_start = None if seg_start is None else np.ascontiguousarray(seg_start, dtype=np.int64)

@@ -7,7 +7,8 @@ each real CLR with the pooled null CLRs.  This module does that bookkeeping (DES
 
   * every replicate is read with ``InputData`` under the run's flags and keeps the ``minCount`` it derives
     (it enters the selection tables' normalisation, v1:399-433);
-  * classes are keyed (k, n, minCount); G and P come from the run's spectrum, the selection rows from one
+  * classes are keyed (k, n, minCount), and (k, n, minCount, bin) in a binned run (bins.py: a replicate's sites
+    are binned by the map lines that name its file name); G and P come from the run's spectrum, the selection rows from one
     ``NormalizedBetaBinom`` per distinct minCount, so every row has the bits a standalone run would build;
   * every replicate is planned with the run's window flags, gap rows are dropped and the windows are offset to
     the replicate's segment of one segmented problem (blmx_load_segmented), scanned in one call;
@@ -27,6 +28,7 @@ import numpy as np
 
 from . import windows
 from .inputs import InputData
+from .bins import BinnedNeutral, binned_classes
 from .native import ScanProblem
 from .neutral import site_classes
 from .problem import GridOrder
@@ -97,17 +99,23 @@ def read_replicates(paths, nofreq, MAF, nosub, minCount, phys, Rrate):
 def null_problem(reps, names, neutral, grids, nofreq, MAF, nosub):
     """One segmented problem of all replicates -> (ScanProblem with seg_start, GridOrder)."""
     order = GridOrder(grids)
-    per = [site_classes(d.count, d.total) for d in reps]
-    for (ck, cn, _), name in zip(per, names):
-        _held(lambda: neutral.class_tables(ck, cn), name, quiet=False)      # the run's message + exit
+    if isinstance(neutral, BinnedNeutral):          # a replicate's sites are binned by the map lines of its name
+        per = [binned_classes(d.count, d.total, neutral.site_bins(os.path.basename(name), d.position))
+               for d, name in zip(reps, names)]
+    else:
+        per = [site_classes(d.count, d.total) for d in reps]
+        per = [(ck, cn, np.zeros(len(ck), np.int64), c) for ck, cn, c in per]
+    for (ck, cn, cb, _), name in zip(per, names):
+        _held(lambda: neutral.class_tables(ck, cn, cb) if cb.any() else neutral.class_tables(ck, cn), name,
+              quiet=False)                                                  # the run's message + exit
     mins = [int(d.minCount) for d in reps]
-    # classes keyed (minCount, n, k)
-    keys = np.concatenate([np.column_stack((np.full(len(ck), m, np.int64), cn, ck))
-                           for (ck, cn, _), m in zip(per, mins)])
+    # classes keyed (minCount, bin, n, k)
+    keys = np.concatenate([np.column_stack((np.full(len(ck), m, np.int64), cb, cn, ck))
+                           for (ck, cn, cb, _), m in zip(per, mins)])
     uniq, inv = np.unique(keys, axis=0, return_inverse=True)
     inv = inv.reshape(-1)
-    cm, cn_all, ck_all = uniq[:, 0], uniq[:, 1], uniq[:, 2]
-    G, P = neutral.class_tables(ck_all, cn_all)
+    cm, cb_all, cn_all, ck_all = uniq[:, 0], uniq[:, 1], uniq[:, 2], uniq[:, 3]
+    G, P = neutral.class_tables(ck_all, cn_all, cb_all) if cb_all.any() else neutral.class_tables(ck_all, cn_all)
     # selection rows: one table per distinct minCount, over that minCount's classes
     own = {m: d.minCount for d, m in zip(reps, mins)}              # a replicate's own minCount object
     rows = {(x, a): np.empty(len(uniq)) for x in order.x for a in order.a}
@@ -126,8 +134,8 @@ def null_problem(reps, names, neutral, grids, nofreq, MAF, nosub):
             r += 1
     sizes = np.array([d.numSites for d in reps], dtype=np.int64)
     seg_start = np.concatenate(([0], np.cumsum(sizes)[:-1])).astype(np.int64)
-    offs = np.concatenate(([0], np.cumsum([len(ck) for ck, _, _ in per])))
-    cls = np.concatenate([inv[offs[i] + c] for i, (_, _, c) in enumerate(per)]).astype(np.int32)
+    offs = np.concatenate(([0], np.cumsum([len(ck) for ck, _, _, _ in per])))
+    cls = np.concatenate([inv[offs[i] + c] for i, (_, _, _, c) in enumerate(per)]).astype(np.int32)
     genpos = np.concatenate([d.genPos for d in reps])
     prob = ScanProblem(genpos, cls, G, SP, np.array([float(v) for v in order.A]), len(order.x), len(order.a),
                        seg_start=seg_start)

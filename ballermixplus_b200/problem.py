@@ -7,10 +7,14 @@ on the site only through its (k, n) class, so the device gets one row per class:
   SP[xa][c]  = NormalizedBetaBinom.get(x, a) * NeutralSFS.propSizes        (v1:479,492)
 with x, a (and A) in the iteration order of the reference's ``set(...)`` loops
 (v1:453,473,474), which is what decides exact ties.
+
+A binned run (bins.py: ``data.siteBin`` and a ``BinnedNeutral``) keys the classes (k, n, bin): G and P come from the
+bin's spectrum, the selection row of the class's (k, n), multiplied by the class's P.
 """
 import numpy as np
 
 from .native import ScanProblem
+from .bins import binned_classes
 from .neutral import site_classes
 
 
@@ -36,6 +40,8 @@ class GridOrder:
 def build_problem(data, neutral, sel, grids):
     """-> (ScanProblem, GridOrder)."""
     order = GridOrder(grids)
+    if getattr(data, 'siteBin', None) is not None:
+        return build_binned(data, neutral, sel, order)
     class_k, class_n, cls = site_classes(data.count, data.total)
     pairs = list(zip(class_k.tolist(), class_n.tolist()))
     if hasattr(neutral, 'class_tables'):
@@ -59,4 +65,32 @@ def build_problem(data, neutral, sel, grids):
             r += 1
     prob = ScanProblem(data.genPos, cls, G, SP, np.array([float(v) for v in order.A]),
                        len(order.x), len(order.a))
+    return prob, order
+
+
+def binned_layout(data, neutral, sel):
+    """Classes keyed (k, n, bin) -> (cls int32[N], G[C], P[C], sel_class int64[C]): sel_class[c] is the index of
+    class c's (k, n) among the selection tables' classes."""
+    ck, cn, cb, cls = binned_classes(data.count, data.total, data.siteBin)
+    G, P = neutral.class_tables(ck, cn, cb)
+    kmax = int(max(ck.max(), sel.class_k.max())) + 1 if len(ck) else 1
+    sel_key = sel.class_n * kmax + sel.class_k            # ascending: site_classes sorts by (n, k)
+    sel_class = np.searchsorted(sel_key, cn * kmax + ck)
+    if len(ck) and not np.array_equal(sel_key[np.minimum(sel_class, len(sel_key) - 1)], cn * kmax + ck):
+        raise ValueError('selection tables were built for different data')
+    return cls, G, P, sel_class
+
+
+def build_binned(data, neutral, sel, order):
+    """``build_problem`` of a binned run -> (ScanProblem, GridOrder); the problem keeps ``layout`` = (P,
+    sel_class) for the fine rows of refine.py."""
+    cls, G, P, sel_class = binned_layout(data, neutral, sel)
+    SP = np.empty((len(order.x) * len(order.a), len(G)), dtype=np.float64)
+    r = 0
+    for x in order.x:
+        for a in order.a:
+            SP[r] = sel.classProbs[(x, a)][sel_class] * P
+            r += 1
+    prob = ScanProblem(data.genPos, cls, G, SP, np.array([float(v) for v in order.A]), len(order.x), len(order.a))
+    prob.layout = (P, sel_class)
     return prob, order

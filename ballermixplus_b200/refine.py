@@ -88,9 +88,11 @@ class RefineGrid:
         return out
 
 
-def fine_tables(grid, boxes, neutral, sel):
+def fine_tables(grid, boxes, neutral, sel, layout=None):
     """Class rows at the fine (x, a) points the boxes need -> (row_of int32 [n_fx * n_fa], SP [n_rows, C]).
-    row_of[fx * n_fa + fa] is the row of SP of that point, or -1; SP = rows * propSizes as build_problem forms it."""
+    row_of[fx * n_fa + fa] is the row of SP of that point, or -1; SP = rows * propSizes as build_problem forms it.
+    ``layout`` (a binned problem's (P, sel_class), problem.build_binned): the classes are the problem's (k, n, bin)
+    classes, each the selection row of its (k, n) times its bin's P."""
     n_fx, n_fa = len(grid.x), len(grid.a)
     need = np.zeros((n_fx, n_fa), bool)
     for b in np.unique(np.asarray(boxes)[:, 2:], axis=0):
@@ -98,8 +100,11 @@ def fine_tables(grid, boxes, neutral, sel):
     idx = np.flatnonzero(need.ravel())
     row_of = np.full(n_fx * n_fa, -1, np.int32)
     row_of[idx] = np.arange(len(idx), dtype=np.int32)
-    _, P = neutral.class_tables(sel.class_k, sel.class_n)
     rows = sel.rows_at([(grid.x[q // n_fa], grid.a[q % n_fa]) for q in idx])
+    if layout is not None:
+        P, sel_class = layout
+        return row_of, rows[:, sel_class] * P[None, :]
+    _, P = neutral.class_tables(sel.class_k, sel.class_n)
     return row_of, rows * P[None, :]
 
 
@@ -116,7 +121,7 @@ def refine_rows(dev, neutral, sel, K, t, lo, hi, iA, ix, ia):
     live = np.flatnonzero(np.asarray(iA) >= 0)
     if len(live):
         boxes = grid.boxes(iA[live], ix[live], ia[live])
-        row_of, SP = fine_tables(grid, boxes, neutral, sel)
+        row_of, SP = fine_tables(grid, boxes, neutral, sel, dev.problem.layout)
         dev.load_refine(np.array([float(v) for v in grid.A]), len(grid.x), len(grid.a), row_of, SP)
         got = dev.refine(t[live], lo[live], hi[live], boxes)
         for col, v in zip((T, fA, fx, fa, ns), got):

@@ -7,7 +7,7 @@ listing for instruction listing (cuobjdump -sass), with scan_kernel<J, GROUP, FA
 scan_kernel<J, GROUP, FAR, SURF> of OLD (before the SPLIT flag) with scan_kernel<J, GROUP, FAR, SURF, SPLIT = false>;
 a kernel OLD already has with the SPLIT flag is compared with the same instantiation in NEW.  Build both with the
 same nvcc flags.  bound_kernel, which the scan runs before scan_kernel, and reduce_kernel, which runs after it, are
-compared as well.  Exit status 1 if any listing differs.
+compared as well; a bound_kernel of OLD without the SLABS flag is compared with bound_kernel<SLABS = 0> of NEW.  Exit status 1 if any listing differs.
 """
 import re
 import subprocess
@@ -40,8 +40,10 @@ def main():
         same += ok
         print(f'{"identical" if ok else "DIFFERENT"}  {name} -> {twin}  ({len(old[name].splitlines())} lines)')
     print(f'{same}/{len(old)} identical')
-    old_b, new_b = ({**scan_kernels(so, 'bound_kernel('), **scan_kernels(so, 'reduce_kernel(')}
-                    for so in sys.argv[1:3])
+    old_b, new_b = ({**scan_kernels(so, 'bound_kernel('), **scan_kernels(so, 'bound_kernel<'),
+                     **scan_kernels(so, 'reduce_kernel(')} for so in sys.argv[1:3])
+    if 'bound_kernel<0>' in new_b:
+        new_b.setdefault('bound_kernel(', new_b['bound_kernel<0>'])
     same_b = sum(old_b[k] == new_b.get(k) for k in old_b)
     for k in sorted(old_b):
         print(f'{"identical" if old_b[k] == new_b.get(k) else "DIFFERENT"}  {k}  ({len(old_b[k].splitlines())} lines)')
